@@ -23,6 +23,7 @@ BASELINE.json configs (one JSON line each, same keys).
              cores, and the measured worth of the visible cores.
 
 `--impl reference` times the CPU oracle instead (all usable host threads), same config.
+`--dump-outputs DIR` writes the result planes of the last timed step as .npy files (dump_outputs).
 """
 from __future__ import annotations
 
@@ -184,6 +185,42 @@ def config_dict(world, desc, works, exchange, planes):
         "exchange": EXCHANGE_TEXT.get(exchange, exchange),
     })
     return c
+
+
+DUMP_PLANES = (("dist", "dist"), ("hops", "hops"), ("first_parent", "fp"), ("n_parents", "npar"), ("nh_mask", "nh"))
+DUMP_BYTES = 64_000_000         # all files of one --dump-outputs run, .npy headers included
+NPY_HEADER_BYTES = 4096         # per graph: 8 files of 128-byte headers, with room to spare
+
+
+def dump_outputs(out_dir, works, lay, buf, bpv, prefix="", budget=DUMP_BYTES):
+    """Write the result planes one timed step left in `buf` (what the device-pointer call hands its
+    caller) as DIR/<prefix><plane>.npy, prefixed g<i>_ as well when the step runs several graphs.
+    16-bit planes become float32 and 32-bit ones float64; a 64-bit plane becomes two float64 planes,
+    <plane> with its low and <plane>_hi with its high 32 bits, so every value is exact.  The files
+    take at most `budget` bytes: when all jobs would not fit, the rows are a fixed, seeded sample of
+    the jobs; job_index.npy names them."""
+    import torch
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    per_graph = budget // len(works) - NPY_HEADER_BYTES
+    for i, (w, o) in enumerate(zip(works, lay)):
+        V, n = w.csr.n_vertices, w.n
+        row_bytes = V * sum({2: 4, 4: 8, 8: 16}[bpv[k]] for _, k in DUMP_PLANES) + 16   # + job_status, job_index
+        k = min(n, per_graph // row_bytes)
+        rows = np.arange(n) if k == n else np.sort(np.random.default_rng(i).choice(n, k, replace=False))
+        sel = torch.from_numpy(rows).to(buf.device)
+        pre = prefix + (f"g{i}_" if len(works) > 1 else "")
+        for name, key in DUMP_PLANES:
+            b = bpv[key]
+            a = buf[o[key]: o[key] + n * V * b].view(n, V * b).index_select(0, sel).cpu().numpy()
+            a = a.view({2: np.uint16, 4: np.uint32, 8: np.uint64}[b])
+            if b == 8:
+                np.save(out / f"{pre}{name}_hi.npy", (a >> np.uint64(32)).astype(np.float64))
+                a = a & np.uint64(0xFFFFFFFF)
+            np.save(out / f"{pre}{name}.npy", a.astype(np.float32 if b == 2 else np.float64))
+        status = buf[o["status"]: o["status"] + 4 * n].cpu().numpy().view(np.uint32)[rows]
+        np.save(out / f"{pre}job_status.npy", status.astype(np.float64))
+        np.save(out / f"{pre}job_index.npy", rows.astype(np.float64))
 
 
 def exchange_note(xchg_bytes, tot):
@@ -558,6 +595,9 @@ def run_ours(args):
     # no exchange: the L2 flush between steps is untimed (sum of per-step kernel events); with an
     # exchange: the whole pipelined region (kernels + exchanges), no flush needed (see config.l2)
     total_ms = float(sum(kern_ms)) if exchange == "none" else float(t_begin.elapsed_time(t_end))
+    if args.dump_outputs:     # every rank its own jobs' planes; together they are the whole step's output
+        dump_outputs(args.dump_outputs, works, lay, bufs[(args.steps - 1) % n_buf], bpv,
+                     prefix=f"r{rank}_" if world > 1 else "", budget=DUMP_BYTES // world)
 
     # ---- e2e: host-pointer C-ABI call, pinned host buffers ----------------------------------
 
@@ -610,7 +650,7 @@ def run_ours(args):
                 if rc != 0:
                     raise RuntimeError(f"host-pointer call rc={rc}: {ctx.last_error()}")
 
-        n_e2e = max(3, min(args.steps, 10))
+        n_e2e = args.steps
         for _ in range(2):
             step()
         barrier()
@@ -646,7 +686,7 @@ def run_ours(args):
     if args.config == "C5" and rank == 0:
         from holo_b200 import ospfv2
         area = desc["_area"]
-        k = 4
+        k = args.steps
         ospfv2.run_area(ctx, area)
         t0 = time.perf_counter()
         for _ in range(k):
@@ -781,7 +821,15 @@ def main():
                          "(distance, hops, next-hop set + job status) or all five planes")
     ap.add_argument("--delta", type=int, default=0, help="SSSP bucket width (tuning; 0 = library default)")
     ap.add_argument("--jobs", type=int, default=JOBS_PER_GPU, help="SPF roots per GPU per step (tuning; BASELINE: 1000)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result planes of the last one as DIR/<plane>.npy in "
+                         "float32 / float64 (r<rank>_<plane>.npy with several GPUs), at most 64,000,000 bytes in all "
+                         "(a seeded sample of the jobs), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm keeps no result planes)")
     DELTA = args.delta
     JOBS_PER_GPU = args.jobs
     if args.warmup < 3 and args.impl == "ours":
