@@ -8,6 +8,7 @@ missing the import fails loudly — there is no Python/CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
+from contextlib import contextmanager
 from dataclasses import dataclass
 from pathlib import Path
 
@@ -39,6 +40,7 @@ JS_INTERNAL = 0x10
 JS_NARROW = 0x20
 RUN_DEVICE_PTRS = 0x1
 MAX_OVERRIDES = 8
+PATHS = {"auto": 0, "general": 1, "general_kahn": 2}   # hspf_debug_set_path
 
 _u32p = C.POINTER(C.c_uint32)
 _u16p = C.POINTER(C.c_uint16)
@@ -104,7 +106,7 @@ EXPORTS = [
     "hspf_xchg_push", "hspf_xchg_wait", "hspf_xchg_release", "hspf_xchg_consumer_stream", "hspf_xchg_sync",
     "hspf_xchg_last_error", "hspf_xchg_destroy", "hspf_xchg_attach_ptr", "hspf_xchg_base", "hspf_xchg_set_push_bytes",
     "hspf_xchg_acquire_direct", "hspf_xchg_peer_deltas", "hspf_xchg_publish", "hspf_ctx_set_peer_slots",
-    "hspf_graph_update_costs",
+    "hspf_graph_update_costs", "hspf_debug_set_path",
 ]
 
 
@@ -150,6 +152,7 @@ def load_library(path: Path | None = None) -> C.CDLL:
     lib.hspf_debug_quad_image.argtypes = [C.POINTER(CsrStruct), C.POINTER(C.c_uint32), _u32p, _u32p, _u16p, _u16p,
                                           _u32p, _u32p, _u32p, _u32p]
     lib.hspf_debug_phase_profile.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint64)]
+    lib.hspf_debug_set_path.argtypes = [C.c_void_p, C.c_int]
     lib.hspf_run_batch16.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(JobsStruct), C.POINTER(Result16Struct), C.c_uint32]
     lib.hspf_run_batch16_async.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(JobsStruct), C.POINTER(Result16Struct)]
     lib.hspf_graph_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint32)]
@@ -370,6 +373,16 @@ class Context:
         self.lib.hspf_ctx_set_peer_slots.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_int64)]
         arr = (C.c_int64 * max(len(deltas), 1))(*deltas)
         self._check(self.lib.hspf_ctx_set_peer_slots(self.handle, len(deltas), arr))
+
+    @contextmanager
+    def path(self, name: str):
+        """Test aid: the batches of the `with` block run on one kernel path (hspf_debug_set_path):
+        "auto" (the default), "general" or "general_kahn"."""
+        self._check(self.lib.hspf_debug_set_path(self.handle, PATHS[name]))
+        try:
+            yield
+        finally:
+            self._check(self.lib.hspf_debug_set_path(self.handle, PATHS["auto"]))
 
     def reserve_sms(self, n_sms: int):
         self._check(self.lib.hspf_ctx_reserve_sms(self.handle, n_sms))

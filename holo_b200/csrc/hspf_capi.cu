@@ -4,11 +4,9 @@
 // There is no CPU compute path in this file: every result plane is produced by
 // spf_batch_kernel on the device.
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <new>
-#include <numeric>
 #include <string>
 #include <vector>
 
@@ -25,12 +23,13 @@ using namespace hspf;
 struct hspf_graph {
     DevGraph d{};
     void *blob = nullptr;      // single device allocation holding every array
-    size_t blob_bytes = 0;
     uint32_t max_indeg = 0;
     bool has_leaf = false;     // any HSPF_VF_LEAF / LEAF_UNLESS_ROOT vertex
-    bool has_quads = false;    // quad-space image present (spf_quad_kernel eligible, see quad_layout.h)
+    bool has_quads = false;    // quad-space image present (see quad_layout.h)
+    bool fast = false;         // spf_quad_kernel serves this graph (decided once, at upload)
     QuadDev q{};
-    std::string quad_why;      // why the quad image was not built
+    QuadLayout qlay{};         // its shared-memory layout
+    std::string why_not_fast;
     // host copies hspf_graph_update_costs validates against
     std::vector<uint32_t> h_row;
     std::vector<uint8_t> h_vflags;
@@ -39,7 +38,7 @@ struct hspf_graph {
 struct hspf_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
-    cudaStream_t copy_stream = nullptr;   // D2H of finished chunks (host-pointer mode)
+    cudaStream_t copy_stream = nullptr;   // D2H of finished jobs (host-pointer mode)
     cudaEvent_t chunk_done = nullptr;
     int sm_count = 0;
     size_t smem_optin = 0;
@@ -53,7 +52,8 @@ struct hspf_ctx {
     void *scratch = nullptr; size_t scratch_bytes = 0;  // planes the caller did not ask for
     unsigned long long *d_prof = nullptr; int prof_rows = 0;  // optional phase counters (debug)
     bool prof_enabled = false;
-    // progress counters of the pipelined host-pointer call (see run_any)
+    int path = HSPF_PATH_AUTO;                // hspf_debug_set_path
+    // progress counters of the pipelined host-pointer call (see run_host)
     uint32_t *d_done = nullptr;               // [kMaxDoneChunks]
     uint32_t *prog_done = nullptr;            // set around one enqueue: the launch publishes per-chunk completion
     uint32_t prog_chunk = 0;
@@ -95,75 +95,60 @@ int grow(hspf_ctx *ctx, void **p, size_t *have, size_t need, bool pinned = false
     return HSPF_OK;
 }
 
-template <typename VT, bool S, bool F>
-int launch(hspf_ctx *ctx, const BatchArgs &args, size_t smem, int grid) {
-    if (const char *co = getenv("HSPF_SMEM_CARVEOUT")) {   // tuning knob (experiments only)
-        CK(cudaFuncSetAttribute(spf_batch_kernel<VT, S, F>, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(co)));
-    }
-    if (smem > 0) {
-        CK(cudaFuncSetAttribute(spf_batch_kernel<VT, S, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    }
-    spf_batch_kernel<VT, S, F><<<grid, kThreads, smem, ctx->stream>>>(args);
-    CK(cudaGetLastError());
-    ctx->launches++;
-    return HSPF_OK;
-}
-
-template <typename VT, bool S>
-int max_ctas_per_sm(size_t smem) {
-    int n = 0;
-    if (smem > 0)
-        cudaFuncSetAttribute(spf_batch_kernel<VT, S, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, spf_batch_kernel<VT, S, false>, kThreads, smem) != cudaSuccess) n = 1;
-    return n < 1 ? 1 : n;
-}
-
 // Result planes of either width: hspf_result (dist u32, first_parent u32, nh_mask u64 x nh_words)
 // or hspf_result16 (all planes u16, one next-hop word of 16 atoms).
+enum Plane { kDist, kHops, kFp, kNpar, kNh, kStatus, kPlanes };   // vertex planes, then the job status
+
 struct AnyResult {
-    void *dist = nullptr;
-    uint16_t *hops = nullptr;
-    void *fp = nullptr;
-    uint16_t *npar = nullptr;
-    void *nh = nullptr;
+    void *p[kPlanes] = {};
+    size_t bytes[kPlanes] = {};   // per vertex of a job; kStatus: per job
     uint32_t nh_words = 1;
-    uint32_t *job_status = nullptr;
     bool narrow = false;
-    size_t dist_b() const { return narrow ? 2 : 4; }
-    size_t fp_b() const { return narrow ? 2 : 4; }
-    size_t nh_b() const { return narrow ? 2 : 8 * (size_t)nh_words; }
 };
 
 AnyResult any_of(const hspf_result *r) {
-    AnyResult a;
-    a.dist = r->dist; a.hops = r->hops; a.fp = r->first_parent; a.npar = r->n_parents; a.nh = r->nh_mask;
-    a.nh_words = r->nh_words; a.job_status = r->job_status; a.narrow = false;
-    return a;
+    return {{r->dist, r->hops, r->first_parent, r->n_parents, r->nh_mask, r->job_status},
+            {4, 2, 4, 2, 8 * (size_t)r->nh_words, 4}, r->nh_words, false};
 }
 
 AnyResult any_of(const hspf_result16 *r) {
-    AnyResult a;
-    a.dist = r->dist; a.hops = r->hops; a.fp = r->first_parent; a.npar = r->n_parents; a.nh = r->nh_mask;
-    a.nh_words = 1; a.job_status = r->job_status; a.narrow = true;
-    return a;
+    return {{r->dist, r->hops, r->first_parent, r->n_parents, r->nh_mask, r->job_status}, {2, 2, 2, 2, 2, 4}, 1, true};
 }
 
-template <int T, bool O>
-int launch_quad(hspf_ctx *ctx, const QuadArgs &args, size_t smem, int per_sm_cap) {
-    CK(cudaFuncSetAttribute(spf_quad_kernel<T, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CK(cudaFuncSetAttribute(spf_quad_kernel<T, O>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, spf_quad_kernel<T, O>, T, smem));
-    if (per_sm < 1) return fail(ctx, HSPF_E_CUDA, "spf_quad_kernel does not fit an SM");
-    if (per_sm_cap > 0 && per_sm > per_sm_cap) per_sm = per_sm_cap;
-    int grid = (ctx->sm_count - ctx->reserved_sms) * per_sm;
-    if (const char *mg = getenv("HSPF_MAX_GRID")) {   // tuning knob (experiments only)
-        int v = atoi(mg);
-        if (v >= 1 && v < grid) grid = v;
+// Points every null plane of `r` at its own 256-byte aligned region of a buffer at `base`, for n_jobs
+// jobs of V vertices, and returns the bytes those regions take (base == nullptr: only counts).
+size_t place_planes(AnyResult &r, uint32_t n_jobs, uint32_t V, uint8_t *base) {
+    size_t used = 0;
+    for (int k = 0; k < kPlanes; ++k) {
+        if (r.p[k]) continue;
+        if (base) r.p[k] = base + used;
+        used += align_up((k == kStatus ? 1 : (size_t)V) * n_jobs * r.bytes[k], 256);
     }
-    if ((uint32_t)grid > args.n_jobs) grid = (int)args.n_jobs;
+    return used;
+}
+
+// Does spf_quad_kernel run this batch?  Decides enqueue's kernel and run_host's pipelined copy.
+bool quad_runs(const hspf_ctx *ctx, const hspf_graph *g, const AnyResult &out) {
+    return g->fast && out.nh_words == 1 && ctx->path == HSPF_PATH_AUTO;
+}
+
+// CTAs of `kernel` one SM holds with `smem` bytes of dynamic shared memory (0 when the query fails).
+template <typename Args>
+int ctas_per_sm(void (*kernel)(Args), int threads, size_t smem) {
+    int n = 0;
+    if (smem > 0) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem) != cudaSuccess) n = 0;
+    return n;
+}
+
+// Grid of a persistent launch, whose CTAs fetch jobs from ctx->d_counter: per_sm CTAs on every SM the
+// ctx does not reserve, at most one per job.  Enqueues the reset of the job counter and, when
+// profiling, of the phase counters (*prof) the launch adds to.
+int begin_launch(hspf_ctx *ctx, int per_sm, uint32_t n_jobs, int &grid, unsigned long long *&prof) {
+    grid = (ctx->sm_count - ctx->reserved_sms) * per_sm;
+    if ((uint32_t)grid > n_jobs) grid = (int)n_jobs;
     if (grid < 1) grid = 1;
-    QuadArgs a = args;
+    prof = nullptr;
     if (ctx->prof_enabled) {
         if (ctx->prof_rows < grid) {
             if (ctx->d_prof) cudaFree(ctx->d_prof);
@@ -172,337 +157,262 @@ int launch_quad(hspf_ctx *ctx, const QuadArgs &args, size_t smem, int per_sm_cap
             ctx->prof_rows = grid;
         }
         CK(cudaMemsetAsync(ctx->d_prof, 0, (size_t)ctx->prof_rows * 16 * sizeof(unsigned long long), ctx->stream));
-        a.prof = ctx->d_prof;
+        prof = ctx->d_prof;
     }
     CK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(uint32_t), ctx->stream));
-    spf_quad_kernel<T, O><<<grid, T, smem, ctx->stream>>>(a);
+    return HSPF_OK;
+}
+
+template <typename Args>
+int start(hspf_ctx *ctx, void (*kernel)(Args), int grid, int threads, size_t smem, const Args &a) {
+    if (smem > 0) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, threads, smem, ctx->stream>>>(a);
     CK(cudaGetLastError());
     ctx->launches++;
     return HSPF_OK;
 }
 
-// The fast path: quad-space kernel (spf_quad.cuh).  Returns 1 if the batch is not eligible.
-int enqueue_quad(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult *out) {
-    if (!g->has_quads || g->has_leaf || (g->d.flags & HSPF_GF_HOPCOUNT) || out->nh_words != 1) return 1;
-    if (getenv("HSPF_NO_QUAD")) return 1;             // tuning knob (experiments only)
-    uint32_t qcap = 2048;
-    if (const char *qc = getenv("HSPF_QUAD_QCAP")) { int v = atoi(qc); if (v >= 64 && v <= 32768) qcap = (uint32_t)v; }
-    int T = 512, cap = 0;
-    if (const char *t = getenv("HSPF_QUAD_T")) T = atoi(t);                 // tuning knobs (experiments only)
-    if (T != 128 && T != 256 && T != 384 && T != 512) T = 512;
-    if (const char *c = getenv("HSPF_CTAS_PER_SM")) cap = atoi(c);
-    const QuadLayout lay = make_quad_layout(g->d.V, g->q.NQ, qcap, (uint32_t)T);
-    if ((size_t)lay.total + 2048 > ctx->smem_optin) return 1;
-    QuadArgs a{};
-    a.g = g->d; a.q = g->q; a.lay = lay;
-    a.n_jobs = jobs->n_jobs; a.roots = jobs->roots;
-    a.ov_off = jobs->ov_off; a.ov_edge = jobs->ov_edge; a.ov_cost = jobs->ov_cost;
-    a.out_dist = static_cast<uint32_t *>(out->dist); a.out_hops = out->hops;
-    a.out_fp = static_cast<uint32_t *>(out->fp); a.out_npar = out->npar;
-    a.out_nh = static_cast<uint64_t *>(out->nh); a.out_status = out->job_status;
-    a.narrow = out->narrow ? 1u : 0u;
-    a.n_peers = out->narrow ? ctx->n_peer_slots : 0u;
-    for (uint32_t k = 0; k < 7; ++k) a.peer_delta[k] = ctx->peer_delta[k];
-    a.done = ctx->prog_done;
-    a.done_chunk = ctx->prog_chunk ? ctx->prog_chunk : 1u;
-    a.job_counter = ctx->d_counter;
-    a.sub_rounds = 1;
-    if (const char *sr = getenv("HSPF_QUAD_SUB")) { int v = atoi(sr); if (v >= 1 && v <= 8) a.sub_rounds = (uint32_t)v; }   // tuning knob
-    const bool ov = jobs->ov_off != nullptr;
-    switch (T) {
-    case 128: return ov ? launch_quad<128, true>(ctx, a, lay.total, cap) : launch_quad<128, false>(ctx, a, lay.total, cap);
-    case 256: return ov ? launch_quad<256, true>(ctx, a, lay.total, cap) : launch_quad<256, false>(ctx, a, lay.total, cap);
-    case 512: return ov ? launch_quad<512, true>(ctx, a, lay.total, cap) : launch_quad<512, false>(ctx, a, lay.total, cap);
-    default: return ov ? launch_quad<384, true>(ctx, a, lay.total, cap) : launch_quad<384, false>(ctx, a, lay.total, cap);
-    }
-}
-
-// Enqueue one batch.  All pointers in `jobs`/`out` are device pointers here.
-int enqueue(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult *out) {
-    {
-        const int rq = enqueue_quad(ctx, g, jobs, out);
-        if (rq != 1) return rq;
-    }
-    if (out->narrow)
-        return fail(ctx, HSPF_E_UNSUPPORTED, "16-bit result planes need the packed fast path (" +
-                    (g->has_quads ? std::string("LEAF flags / hop-count mode") : g->quad_why) + ")");
-    const uint32_t V = g->d.V;
-    const bool q16 = V <= 0xFFFFu;
-    const Layout lay = make_layout(V, g->d.E, q16 ? 2 : 4);
-    const size_t sb = lay.total;
-    // static smem of the kernel (Small) is ~4.5 KB; leave headroom
-    const size_t smem_cap = ctx->smem_optin > 6144 ? ctx->smem_optin - 6144 : 0;
-    const bool in_smem = sb <= smem_cap;
-
-    BatchArgs a{};
+// The arguments both kernels share: graph, jobs, result planes, job counter.
+template <typename Args>
+Args kernel_args(const hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out) {
+    Args a{};
     a.g = g->d;
-    a.lay = lay;
     a.n_jobs = jobs->n_jobs;
     a.roots = jobs->roots;
     a.ov_off = jobs->ov_off;
     a.ov_edge = jobs->ov_edge;
     a.ov_cost = jobs->ov_cost;
-    a.out_dist = static_cast<uint32_t *>(out->dist);
-    a.out_hops = out->hops;
-    a.out_fp = static_cast<uint32_t *>(out->fp);
-    a.out_npar = out->npar;
-    a.out_nh = static_cast<uint64_t *>(out->nh);
-    a.out_status = out->job_status;
-    a.nhw = out->nh_words;
+    a.out_dist = static_cast<uint32_t *>(out.p[kDist]);
+    a.out_hops = static_cast<uint16_t *>(out.p[kHops]);
+    a.out_fp = static_cast<uint32_t *>(out.p[kFp]);
+    a.out_npar = static_cast<uint16_t *>(out.p[kNpar]);
+    a.out_nh = static_cast<uint64_t *>(out.p[kNh]);
+    a.out_status = static_cast<uint32_t *>(out.p[kStatus]);
     a.job_counter = ctx->d_counter;
+    return a;
+}
+
+// Enqueue one batch.  All pointers in `jobs`/`out` are device pointers here.
+int enqueue(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out) {
+    int grid = 0, rc;
+    if (quad_runs(ctx, g, out)) {   // the fast path, spf_quad.cuh
+        QuadArgs a = kernel_args<QuadArgs>(ctx, g, jobs, out);
+        a.q = g->q;
+        a.lay = g->qlay;
+        a.narrow = out.narrow ? 1u : 0u;
+        a.n_peers = out.narrow ? ctx->n_peer_slots : 0u;
+        for (uint32_t k = 0; k < 7; ++k) a.peer_delta[k] = ctx->peer_delta[k];
+        a.done = ctx->prog_done;
+        a.done_chunk = ctx->prog_chunk ? ctx->prog_chunk : 1u;
+        const auto kernel = jobs->ov_off ? spf_quad_kernel<true> : spf_quad_kernel<false>;
+        CK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        const int per_sm = ctas_per_sm(kernel, kQuadThreads, a.lay.total);
+        if (per_sm < 1) return fail(ctx, HSPF_E_CUDA, "spf_quad_kernel does not fit an SM");
+        if ((rc = begin_launch(ctx, per_sm, jobs->n_jobs, grid, a.prof))) return rc;
+        return start(ctx, kernel, grid, kQuadThreads, a.lay.total, a);
+    }
+    if (out.narrow)
+        return fail(ctx, HSPF_E_UNSUPPORTED, "16-bit result planes need the packed fast path (" +
+                    (g->fast ? std::string("general kernel selected by hspf_debug_set_path") : g->why_not_fast) + ")");
+    const uint32_t V = g->d.V;
+    const bool q16 = V <= 0xFFFFu;
+    BatchArgs a = kernel_args<BatchArgs>(ctx, g, jobs, out);
+    a.lay = make_layout(V, g->d.E, q16 ? 2 : 4);
+    a.nhw = out.nh_words;
+    const size_t sb = a.lay.total;
+    // static smem of the kernel (Small) is ~4.5 KB; leave headroom
+    const size_t smem_cap = ctx->smem_optin > 6144 ? ctx->smem_optin - 6144 : 0;
+    const bool in_smem = sb <= smem_cap;
     // pointer-jumping next-hop phase: needs the aliased layout (dagbit in qa, words over dist)
-    a.jump_ok = (in_smem && q16 && g->d.iedge16 && g->d.edge16 && g->d.iquad && lay.dagbit == lay.qa && lay.kq0 == lay.dist && !getenv("HSPF_NO_JUMP")) ? 1u : 0u;
-    if (getenv("HSPF_NO_ROW16")) a.g.row16 = nullptr;   // tuning knob (experiments only)
-
-    int per_sm = in_smem ? (q16 ? max_ctas_per_sm<uint16_t, true>(sb) : max_ctas_per_sm<uint32_t, true>(sb))
-                         : (q16 ? max_ctas_per_sm<uint16_t, false>(0) : max_ctas_per_sm<uint32_t, false>(0));
-    if (const char *lim = getenv("HSPF_CTAS_PER_SM")) {   // tuning knob (experiments only)
-        int v = atoi(lim);
-        if (v >= 1 && v < per_sm) per_sm = v;
-    }
-    // SMs reserved for a concurrent kernel: launch fewer persistent CTAs (job fetch is dynamic)
-    int grid = (ctx->sm_count - ctx->reserved_sms) * per_sm;
-    if (const char *mg = getenv("HSPF_MAX_GRID")) {   // tuning knob (experiments only)
-        int v = atoi(mg);
-        if (v >= 1 && v < grid) grid = v;
-    }
-    if ((uint32_t)grid > jobs->n_jobs) grid = (int)jobs->n_jobs;
-    if (grid < 1) grid = 1;
-
+    a.jump_ok = (ctx->path != HSPF_PATH_GENERAL_KAHN && in_smem && q16 && g->d.iedge16 && g->d.edge16 && g->d.iquad &&
+                 a.lay.dagbit == a.lay.qa && a.lay.kq0 == a.lay.dist) ? 1u : 0u;
+    // the grid is sized for the variant without the no-override specialisation
+    using Kernel = void (*)(BatchArgs);
+    const Kernel general = in_smem ? (q16 ? spf_batch_kernel<uint16_t, true, false> : spf_batch_kernel<uint32_t, true, false>)
+                                   : (q16 ? spf_batch_kernel<uint16_t, false, false> : spf_batch_kernel<uint32_t, false, false>);
+    const bool fast = in_smem && !jobs->ov_off && !(g->d.flags & HSPF_GF_HOPCOUNT) && !g->has_leaf && out.nh_words == 1;
+    const Kernel kernel = !fast ? general : q16 ? spf_batch_kernel<uint16_t, true, true> : spf_batch_kernel<uint32_t, true, true>;
+    const size_t smem = in_smem ? sb : 0;
+    if ((rc = begin_launch(ctx, std::max(1, ctas_per_sm(general, kThreads, smem)), jobs->n_jobs, grid, a.prof))) return rc;
     if (!in_smem) {
-        int rc = grow(ctx, &ctx->ws, &ctx->ws_bytes, sb * (size_t)grid);
-        if (rc) return rc;
+        if ((rc = grow(ctx, &ctx->ws, &ctx->ws_bytes, sb * (size_t)grid))) return rc;
         a.ws = static_cast<uint8_t *>(ctx->ws);
         a.ws_stride = sb;
     }
-    if (ctx->prof_enabled) {
-        if (ctx->prof_rows < grid) {
-            if (ctx->d_prof) cudaFree(ctx->d_prof);
-            CK(cudaMalloc(&ctx->d_prof, (size_t)grid * 16 * sizeof(unsigned long long)));
-            ctx->prof_rows = grid;
-        }
-        CK(cudaMemsetAsync(ctx->d_prof, 0, (size_t)ctx->prof_rows * 16 * sizeof(unsigned long long), ctx->stream));
-        a.prof = ctx->d_prof;
-    }
-    CK(cudaMemsetAsync(ctx->d_counter, 0, sizeof(uint32_t), ctx->stream));
-    const bool fast = !jobs->ov_off && !(g->d.flags & HSPF_GF_HOPCOUNT) && !g->has_leaf && out->nh_words == 1;
-    if (in_smem) {
-        if (fast) return q16 ? launch<uint16_t, true, true>(ctx, a, sb, grid) : launch<uint32_t, true, true>(ctx, a, sb, grid);
-        return q16 ? launch<uint16_t, true, false>(ctx, a, sb, grid) : launch<uint32_t, true, false>(ctx, a, sb, grid);
-    }
-    return q16 ? launch<uint16_t, false, false>(ctx, a, 0, grid) : launch<uint32_t, false, false>(ctx, a, 0, grid);
+    return start(ctx, kernel, grid, kThreads, smem, a);
 }
 
-struct Planes {   // byte sizes of the result planes of a batch
-    size_t dist, hops, fp, npar, nh, status;
-    size_t total() const { return dist + hops + fp + npar + nh + status; }
-};
-
-Planes plane_sizes(uint32_t n_jobs, uint32_t V, const AnyResult &r) {
-    auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-    size_t n = (size_t)n_jobs * V;
-    Planes p;
-    p.dist = al(n * r.dist_b()); p.hops = al(n * 2); p.fp = al(n * r.fp_b()); p.npar = al(n * 2);
-    p.nh = al(n * r.nh_b()); p.status = al((size_t)n_jobs * 4);
-    return p;
+// Device-pointer call.
+int run_device(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out) {
+    // planes the caller skipped still have to exist on the device
+    AnyResult r = out;
+    if (const size_t need = place_planes(r, jobs->n_jobs, g->d.V, nullptr)) {
+        if (const int rc = grow(ctx, &ctx->scratch, &ctx->scratch_bytes, need)) return rc;
+        place_planes(r, jobs->n_jobs, g->d.V, static_cast<uint8_t *>(ctx->scratch));
+    }
+    return enqueue(ctx, g, jobs, r);
 }
 
-int check_result_args(hspf_ctx *ctx, const AnyResult &out) {
-    if (out.nh_words < 1 || out.nh_words > 4) return fail(ctx, HSPF_E_INVAL, "nh_words must be 1..4");
+// D2H on the copy stream: jobs [j0, j0 + nj) of every vertex plane the caller asked for.
+int copy_out(hspf_ctx *ctx, const AnyResult &host, const AnyResult &dev, uint32_t V, uint32_t j0, uint32_t nj) {
+    for (int k = 0; k < kStatus; ++k) {
+        if (!host.p[k]) continue;
+        const size_t o = (size_t)j0 * V * host.bytes[k];
+        CK(cudaMemcpyAsync(static_cast<uint8_t *>(host.p[k]) + o, static_cast<uint8_t *>(dev.p[k]) + o,
+                           (size_t)nj * V * host.bytes[k], cudaMemcpyDeviceToHost, ctx->copy_stream));
+    }
     return HSPF_OK;
 }
 
-int run_async_any(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out);
-int run_any(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out, uint32_t flags);
-
-int run_async_any(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out) {
-    int rc = check_result_args(ctx, out);
-    if (rc) return rc;
-    if (jobs->n_jobs == 0) return HSPF_OK;
-    if (!jobs->roots) return fail(ctx, HSPF_E_INVAL, "null roots");
-    try {
-        CK(cudaSetDevice(ctx->device));
-        // planes the caller skipped still have to exist on the device
-        AnyResult r = out;
-        Planes ps = plane_sizes(jobs->n_jobs, g->d.V, r);
-        size_t need = 0;
-        if (!r.dist) need += ps.dist;
-        if (!r.hops) need += ps.hops;
-        if (!r.fp) need += ps.fp;
-        if (!r.npar) need += ps.npar;
-        if (!r.nh) need += ps.nh;
-        if (!r.job_status) need += ps.status;
-        if (need) {
-            rc = grow(ctx, &ctx->scratch, &ctx->scratch_bytes, need);
-            if (rc) return rc;
-            uint8_t *p = static_cast<uint8_t *>(ctx->scratch);
-            if (!r.dist) { r.dist = p; p += ps.dist; }
-            if (!r.hops) { r.hops = reinterpret_cast<uint16_t *>(p); p += ps.hops; }
-            if (!r.fp) { r.fp = p; p += ps.fp; }
-            if (!r.npar) { r.npar = reinterpret_cast<uint16_t *>(p); p += ps.npar; }
-            if (!r.nh) { r.nh = p; p += ps.nh; }
-            if (!r.job_status) { r.job_status = reinterpret_cast<uint32_t *>(p); p += ps.status; }
-        }
-        return enqueue(ctx, g, jobs, &r);
-    } catch (...) {
-        return fail(ctx, HSPF_E_INVAL, "unexpected exception");
+// Host image of a device buffer (a graph's blob, a batch's job arrays): sections back to back, each
+// 256-byte aligned, and the pointer fields to aim at them once the buffer has its device address.
+struct BlobImage {
+    std::vector<uint8_t> bytes;
+    std::vector<std::function<void(const uint8_t *)>> bind;
+    // n elements of src (null: the section stays zero); `field` is null unless `used`
+    template <typename F, typename S>
+    void add(const F *&field, const S *src, size_t n, bool used = true) {
+        const size_t o = bytes.size();
+        bytes.resize(o + align_up(n * sizeof(S), 256), 0);
+        if (src && n) std::memcpy(bytes.data() + o, src, n * sizeof(S));
+        field = nullptr;
+        if (used) bind.push_back([&field, o](const uint8_t *b) { field = reinterpret_cast<const F *>(b + o); });
     }
+    template <typename F, typename S>
+    void add(const F *&field, const std::vector<S> &v, bool used = true) { add(field, v.data(), v.size(), used); }
+};
+
+// Host-pointer call: validate the jobs, stage them in, run, stage the planes out.
+int run_host(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out) {
+    const uint32_t n = jobs->n_jobs, V = g->d.V;
+    int rc;
+    uint32_t n_ov = 0;
+    for (uint32_t j = 0; j < n; ++j)
+        if (jobs->roots[j] >= V) return fail(ctx, HSPF_E_INVAL, "root out of range");
+    if (jobs->ov_off) {
+        if (!jobs->ov_edge || !jobs->ov_cost) {
+            if (jobs->ov_off[n] != 0) return fail(ctx, HSPF_E_INVAL, "null override arrays");
+        }
+        for (uint32_t j = 0; j < n; ++j) {
+            if (jobs->ov_off[j + 1] < jobs->ov_off[j]) return fail(ctx, HSPF_E_INVAL, "ov_off not monotone");
+            if (jobs->ov_off[j + 1] - jobs->ov_off[j] > HSPF_MAX_OVERRIDES)
+                return fail(ctx, HSPF_E_UNSUPPORTED, "more than HSPF_MAX_OVERRIDES overrides in a job");
+        }
+        n_ov = jobs->ov_off[n];
+        for (uint32_t i = 0; i < n_ov; ++i)
+            if (jobs->ov_edge[i] >= g->d.E) return fail(ctx, HSPF_E_INVAL, "override edge out of range");
+    }
+    hspf_jobs dj{};
+    dj.n_jobs = n;
+    BlobImage in;
+    in.add(dj.roots, jobs->roots, n);
+    in.add(dj.ov_off, jobs->ov_off, jobs->ov_off ? n + 1 : 0, jobs->ov_off != nullptr);
+    in.add(dj.ov_edge, jobs->ov_edge, n_ov);
+    in.add(dj.ov_cost, jobs->ov_cost, n_ov);
+    const size_t in_total = in.bytes.size();
+    AnyResult dr = out;
+    for (void *&p : dr.p) p = nullptr;
+    const size_t dev_total = in_total + place_planes(dr, n, V, nullptr);
+    rc = grow(ctx, &ctx->stage, &ctx->stage_bytes, dev_total);
+    if (rc) return rc;
+    rc = grow(ctx, &ctx->h_pin, &ctx->h_pin_bytes, in_total, true);
+    if (rc) return rc;
+    uint8_t *dp = static_cast<uint8_t *>(ctx->stage);
+    std::memcpy(ctx->h_pin, in.bytes.data(), in_total);
+    CK(cudaMemcpyAsync(dp, ctx->h_pin, in_total, cudaMemcpyHostToDevice, ctx->stream));
+    for (auto &b : in.bind) b(dp);
+    place_planes(dr, n, V, dp + in_total);
+    // Fast path: ONE launch for the whole batch; the kernel counts finished jobs per piece
+    // (release ordered behind their planes) and the copy stream waits on those counters with
+    // stream memory operations, so a piece's planes travel to the host while the rest of the
+    // batch still computes.  (Launching the batch in pieces instead costs more than it hides:
+    // a launch cannot finish faster than one job's latency.  Measured on B200, C2, 6 B/vertex:
+    // 1 piece 631 k SPF/s, 4 pieces 532 k, 16 pieces 264 k.)  Four pieces: few, large copies,
+    // every cudaMemcpyAsync costs ~10 us here.
+    const bool pipelined = quad_runs(ctx, g, out) && ctx->wait_value && n >= 256;
+    const uint32_t piece = (n + 3) / 4;
+    if (pipelined) {
+        CK(cudaMemsetAsync(ctx->d_done, 0, 64 * sizeof(uint32_t), ctx->stream));
+        CK(cudaEventRecord(ctx->prog_reset, ctx->stream));
+        ctx->prog_done = ctx->d_done; ctx->prog_chunk = piece;
+    }
+    rc = enqueue(ctx, g, &dj, dr);
+    ctx->prog_done = nullptr; ctx->prog_chunk = 0;
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->chunk_done, ctx->stream));
+    cudaStream_t cs = ctx->copy_stream;
+    if (pipelined) {
+        CK(cudaStreamWaitEvent(cs, ctx->prog_reset, 0));       // the counters of this call, not of the last one
+        for (uint32_t c = 0, c0 = 0; c0 < n; ++c, c0 += piece) {
+            const uint32_t cn = std::min(piece, n - c0);
+            if (ctx->wait_value(reinterpret_cast<CUstream>(cs), reinterpret_cast<CUdeviceptr>(ctx->d_done + c), cn,
+                                CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
+                return fail(ctx, HSPF_E_CUDA, "cuStreamWaitValue32 failed");
+            if ((rc = copy_out(ctx, out, dr, V, c0, cn))) return rc;
+        }
+    }
+    CK(cudaStreamWaitEvent(cs, ctx->chunk_done, 0));
+    if (!pipelined && (rc = copy_out(ctx, out, dr, V, 0, n))) return rc;
+    std::vector<uint32_t> st(n);
+    CK(cudaMemcpyAsync(st.data(), dr.p[kStatus], (size_t)n * 4, cudaMemcpyDeviceToHost, cs));
+    CK(cudaStreamSynchronize(cs));
+    CK(cudaStreamSynchronize(ctx->stream));
+    bool any = false;
+    for (uint32_t j = 0; j < n; ++j) any |= (st[j] != 0);
+    if (out.p[kStatus]) std::memcpy(out.p[kStatus], st.data(), (size_t)n * 4);
+    if (any) return fail(ctx, HSPF_E_JOB_STATUS, "one or more jobs need the CPU path (see job_status)");
+    return HSPF_OK;
 }
 
-int run_any(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const AnyResult &out, uint32_t flags) {
-    int rc = check_result_args(ctx, out);
-    if (rc) return rc;
+// The four run calls: shared checks, then the device-pointer call (synchronised unless async) or the
+// host-pointer call.
+template <typename R>
+int run_checked(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const R *out, bool async, uint32_t flags) {
+    if (!ctx || !g || !jobs) return HSPF_E_INVAL;
+    if (!out) return fail(ctx, HSPF_E_INVAL, "null result");
+    const AnyResult r = any_of(out);
+    if (r.nh_words < 1 || r.nh_words > 4) return fail(ctx, HSPF_E_INVAL, "nh_words must be 1..4");
     if (jobs->n_jobs == 0) return HSPF_OK;
     if (!jobs->roots) return fail(ctx, HSPF_E_INVAL, "null roots");
     try {
         CK(cudaSetDevice(ctx->device));
-        const uint32_t n = jobs->n_jobs, V = g->d.V;
-        if (flags & HSPF_RUN_DEVICE_PTRS) {
-            rc = run_async_any(ctx, g, jobs, out);
-            if (rc) return rc;
-            CK(cudaStreamSynchronize(ctx->stream));
-            return HSPF_OK;   // job_status stays on the device in this mode
-        }
-        // ---- host-pointer mode: validate, stage in, run, stage out --------------
-        uint32_t n_ov = 0;
-        for (uint32_t j = 0; j < n; ++j)
-            if (jobs->roots[j] >= V) return fail(ctx, HSPF_E_INVAL, "root out of range");
-        if (jobs->ov_off) {
-            if (!jobs->ov_edge || !jobs->ov_cost) {
-                if (jobs->ov_off[n] != 0) return fail(ctx, HSPF_E_INVAL, "null override arrays");
-            }
-            for (uint32_t j = 0; j < n; ++j) {
-                if (jobs->ov_off[j + 1] < jobs->ov_off[j]) return fail(ctx, HSPF_E_INVAL, "ov_off not monotone");
-                if (jobs->ov_off[j + 1] - jobs->ov_off[j] > HSPF_MAX_OVERRIDES)
-                    return fail(ctx, HSPF_E_UNSUPPORTED, "more than HSPF_MAX_OVERRIDES overrides in a job");
-            }
-            n_ov = jobs->ov_off[n];
-            for (uint32_t i = 0; i < n_ov; ++i)
-                if (jobs->ov_edge[i] >= g->d.E) return fail(ctx, HSPF_E_INVAL, "override edge out of range");
-        }
-        auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-        const size_t in_roots = al((size_t)n * 4);
-        const size_t in_off = jobs->ov_off ? al((size_t)(n + 1) * 4) : 0;
-        const size_t in_ove = al((size_t)n_ov * 4 + 4), in_ovc = al((size_t)n_ov * 4 + 4);
-        const size_t in_total = in_roots + in_off + in_ove + in_ovc;
-        Planes ps = plane_sizes(n, V, out);
-        const size_t dev_total = in_total + ps.total();
-        rc = grow(ctx, &ctx->stage, &ctx->stage_bytes, dev_total);
-        if (rc) return rc;
-        rc = grow(ctx, &ctx->h_pin, &ctx->h_pin_bytes, in_total, true);
-        if (rc) return rc;
-        uint8_t *hp = static_cast<uint8_t *>(ctx->h_pin);
-        uint8_t *dp = static_cast<uint8_t *>(ctx->stage);
-        std::memcpy(hp, jobs->roots, (size_t)n * 4);
-        if (jobs->ov_off) {
-            std::memcpy(hp + in_roots, jobs->ov_off, (size_t)(n + 1) * 4);
-            if (n_ov) {
-                std::memcpy(hp + in_roots + in_off, jobs->ov_edge, (size_t)n_ov * 4);
-                std::memcpy(hp + in_roots + in_off + in_ove, jobs->ov_cost, (size_t)n_ov * 4);
-            }
-        }
-        CK(cudaMemcpyAsync(dp, hp, in_total, cudaMemcpyHostToDevice, ctx->stream));
-        hspf_jobs dj{};
-        dj.n_jobs = n;
-        dj.roots = reinterpret_cast<const uint32_t *>(dp);
-        dj.ov_off = jobs->ov_off ? reinterpret_cast<const uint32_t *>(dp + in_roots) : nullptr;
-        dj.ov_edge = reinterpret_cast<const uint32_t *>(dp + in_roots + in_off);
-        dj.ov_cost = reinterpret_cast<const uint32_t *>(dp + in_roots + in_off + in_ove);
-        uint8_t *rp = dp + in_total;
-        AnyResult dr = out;
-        dr.dist = rp; rp += ps.dist;
-        dr.hops = reinterpret_cast<uint16_t *>(rp); rp += ps.hops;
-        dr.fp = rp; rp += ps.fp;
-        dr.npar = reinterpret_cast<uint16_t *>(rp); rp += ps.npar;
-        dr.nh = rp; rp += ps.nh;
-        dr.job_status = reinterpret_cast<uint32_t *>(rp); rp += ps.status;
-        std::vector<uint32_t> st(n);
-        const size_t db = out.dist_b(), fb = out.fp_b(), nb = out.nh_b();
-        // Fast path: ONE launch for the whole batch; the kernel counts finished jobs per chunk
-        // (release ordered behind their planes) and the copy stream waits on those counters with
-        // stream memory operations, so a chunk's planes travel to the host while the rest of the
-        // batch still computes.  (Launching the batch in pieces instead costs more than it hides:
-        // a launch cannot finish faster than one job's latency.  Measured on B200, C2, 6 B/vertex:
-        // 1 piece 631 k SPF/s, 4 pieces 532 k, 16 pieces 264 k.)
-        const bool quad_ok = g->has_quads && !g->has_leaf && !(g->d.flags & HSPF_GF_HOPCOUNT) && out.nh_words == 1 &&
-                             !getenv("HSPF_NO_QUAD");
-        if (quad_ok && ctx->wait_value && n >= 256 && !getenv("HSPF_E2E_CHUNK")) {
-            uint32_t pieces = 4;       // few, large copies: every cudaMemcpyAsync costs ~10 us here
-            if (const char *pc = getenv("HSPF_E2E_PIECES")) { int v = atoi(pc); if (v >= 1 && v <= 64) pieces = (uint32_t)v; }   // tuning knob
-            const uint32_t pchunk = std::max<uint32_t>(1, (n + pieces - 1) / pieces);
-            const uint32_t n_chunks = (n + pchunk - 1) / pchunk;
-            CK(cudaMemsetAsync(ctx->d_done, 0, 64 * sizeof(uint32_t), ctx->stream));
-            CK(cudaEventRecord(ctx->prog_reset, ctx->stream));
-            ctx->prog_done = ctx->d_done; ctx->prog_chunk = pchunk;
-            rc = enqueue(ctx, g, &dj, &dr);
-            ctx->prog_done = nullptr; ctx->prog_chunk = 0;
-            if (rc) return rc;
-            CK(cudaEventRecord(ctx->chunk_done, ctx->stream));
-            cudaStream_t cs = ctx->copy_stream;
-            CK(cudaStreamWaitEvent(cs, ctx->prog_reset, 0));       // the counters of this call, not of the last one
-            for (uint32_t c = 0; c < n_chunks; ++c) {
-                const uint32_t c0 = c * pchunk, cn = std::min(pchunk, n - c0);
-                if (ctx->wait_value(reinterpret_cast<CUstream>(cs), reinterpret_cast<CUdeviceptr>(ctx->d_done + c), cn,
-                                    CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
-                    return fail(ctx, HSPF_E_CUDA, "cuStreamWaitValue32 failed");
-                const size_t o = (size_t)c0 * V, cv = (size_t)cn * V;
-                if (out.dist) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.dist) + o * db, static_cast<uint8_t *>(dr.dist) + o * db, cv * db, cudaMemcpyDeviceToHost, cs));
-                if (out.hops) CK(cudaMemcpyAsync(out.hops + o, dr.hops + o, cv * 2, cudaMemcpyDeviceToHost, cs));
-                if (out.fp) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.fp) + o * fb, static_cast<uint8_t *>(dr.fp) + o * fb, cv * fb, cudaMemcpyDeviceToHost, cs));
-                if (out.npar) CK(cudaMemcpyAsync(out.npar + o, dr.npar + o, cv * 2, cudaMemcpyDeviceToHost, cs));
-                if (out.nh) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.nh) + o * nb, static_cast<uint8_t *>(dr.nh) + o * nb, cv * nb, cudaMemcpyDeviceToHost, cs));
-            }
-            CK(cudaStreamWaitEvent(cs, ctx->chunk_done, 0));
-            CK(cudaMemcpyAsync(st.data(), dr.job_status, (size_t)n * 4, cudaMemcpyDeviceToHost, cs));
-            CK(cudaStreamSynchronize(cs));
-            CK(cudaStreamSynchronize(ctx->stream));
-            bool any = false;
-            for (uint32_t j = 0; j < n; ++j) any |= (st[j] != 0);
-            if (out.job_status) std::memcpy(out.job_status, st.data(), (size_t)n * 4);
-            if (any) return fail(ctx, HSPF_E_JOB_STATUS, "one or more jobs need the CPU path (see job_status)");
-            return HSPF_OK;
-        }
-        // General path: one launch (HSPF_E2E_CHUNK: pieces, each copied back on a second stream
-        // while the next one computes).
-        uint32_t chunk = n;
-        if (const char *cs = getenv("HSPF_E2E_CHUNK")) { int v = atoi(cs); if (v > 0) chunk = (uint32_t)v; }
-        for (uint32_t c0 = 0; c0 < n; c0 += chunk) {
-            const uint32_t cn = std::min(chunk, n - c0);
-            hspf_jobs cj = dj;
-            cj.n_jobs = cn;
-            cj.roots = dj.roots + c0;
-            if (dj.ov_off) cj.ov_off = dj.ov_off + c0;    // offsets stay absolute into ov_edge/ov_cost
-            AnyResult cr = dr;
-            const size_t o = (size_t)c0 * V;
-            cr.dist = static_cast<uint8_t *>(dr.dist) + o * db; cr.hops = dr.hops + o;
-            cr.fp = static_cast<uint8_t *>(dr.fp) + o * fb; cr.npar = dr.npar + o;
-            cr.nh = static_cast<uint8_t *>(dr.nh) + o * nb;
-            cr.job_status = dr.job_status + c0;
-            rc = enqueue(ctx, g, &cj, &cr);
-            if (rc) return rc;
-            CK(cudaEventRecord(ctx->chunk_done, ctx->stream));
-            CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->chunk_done, 0));
-            const size_t cv = (size_t)cn * V;
-            cudaStream_t cs = ctx->copy_stream;
-            if (out.dist) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.dist) + o * db, cr.dist, cv * db, cudaMemcpyDeviceToHost, cs));
-            if (out.hops) CK(cudaMemcpyAsync(out.hops + o, cr.hops, cv * 2, cudaMemcpyDeviceToHost, cs));
-            if (out.fp) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.fp) + o * fb, cr.fp, cv * fb, cudaMemcpyDeviceToHost, cs));
-            if (out.npar) CK(cudaMemcpyAsync(out.npar + o, cr.npar, cv * 2, cudaMemcpyDeviceToHost, cs));
-            if (out.nh) CK(cudaMemcpyAsync(static_cast<uint8_t *>(out.nh) + o * nb, cr.nh, cv * nb, cudaMemcpyDeviceToHost, cs));
-            CK(cudaMemcpyAsync(st.data() + c0, cr.job_status, (size_t)cn * 4, cudaMemcpyDeviceToHost, cs));
-        }
-        CK(cudaStreamSynchronize(ctx->copy_stream));
+        if (!async && !(flags & HSPF_RUN_DEVICE_PTRS)) return run_host(ctx, g, jobs, r);
+        const int rc = run_device(ctx, g, jobs, r);
+        if (rc || async) return rc;
         CK(cudaStreamSynchronize(ctx->stream));
-        bool any = false;
-        for (uint32_t j = 0; j < n; ++j) any |= (st[j] != 0);
-        if (out.job_status) std::memcpy(out.job_status, st.data(), (size_t)n * 4);
-        if (any) return fail(ctx, HSPF_E_JOB_STATUS, "one or more jobs need the CPU path (see job_status)");
-        return HSPF_OK;
+        return HSPF_OK;   // job_status stays on the device in this mode
     } catch (const std::bad_alloc &) {
         return fail(ctx, HSPF_E_NOMEM, "host allocation failed");
     } catch (...) {
         return fail(ctx, HSPF_E_INVAL, "unexpected exception");
     }
+}
+
+// Transposed CSR: the in-edges of v are src/cost/fwd[irow[v] .. irow[v + 1]), ordered by (source,
+// forward edge index).  col[] must be in range.
+struct Transposed {
+    std::vector<uint32_t> irow, src, cost, fwd;
+};
+
+Transposed transpose(const hspf_csr *g) {
+    const uint32_t V = g->n_vertices, E = g->n_edges;
+    Transposed t;
+    t.irow.assign(V + 1, 0);
+    t.src.resize(E); t.cost.resize(E); t.fwd.resize(E);
+    for (uint32_t e = 0; e < E; ++e) t.irow[g->col[e] + 1]++;
+    for (uint32_t v = 0; v < V; ++v) t.irow[v + 1] += t.irow[v];
+    std::vector<uint32_t> fill(t.irow.begin(), t.irow.end() - 1);
+    for (uint32_t u = 0; u < V; ++u)
+        for (uint32_t e = g->row_ptr[u]; e < g->row_ptr[u + 1]; ++e) {
+            const uint32_t k = fill[g->col[e]]++;
+            t.src[k] = u; t.cost[k] = g->cost[e]; t.fwd[k] = e;
+        }
+    return t;
+}
+
+QuadHost quads_of(const hspf_csr *g, const Transposed &t) {
+    return build_quads(g->n_vertices, g->n_edges, g->row_ptr, g->col, g->cost, g->vflags, t.irow.data(), t.src.data(),
+                       t.cost.data(), t.fwd.data(), g->delta);
 }
 
 }  // namespace
@@ -602,6 +512,12 @@ int hspf_debug_phase_profile(hspf_ctx *ctx, int enable, uint64_t out[16]) {
     return HSPF_OK;
 }
 
+int hspf_debug_set_path(hspf_ctx *ctx, int path) {
+    if (!ctx || path < HSPF_PATH_AUTO || path > HSPF_PATH_GENERAL_KAHN) return HSPF_E_INVAL;
+    ctx->path = path;
+    return HSPF_OK;
+}
+
 int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
     if (!ctx || !g || !out) return HSPF_E_INVAL;
     *out = nullptr;
@@ -612,7 +528,6 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         if (g->row_ptr[0] != 0 || g->row_ptr[V] != E) return fail(ctx, HSPF_E_INVAL, "row_ptr[0]!=0 or row_ptr[V]!=E");
         bool zero_cost_hop_tail = false;
         uint64_t cost_sum = 0;
-        std::vector<uint32_t> indeg(V + 1, 0);
         for (uint32_t u = 0; u < V; ++u) {
             if (g->row_ptr[u + 1] < g->row_ptr[u]) return fail(ctx, HSPF_E_INVAL, "row_ptr not monotone");
             const bool uh = g->vflags[u] & HSPF_VF_HOP;
@@ -624,7 +539,6 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
                 if (!uh && !(g->vflags[v] & HSPF_VF_HOP)) return fail(ctx, HSPF_E_INVAL, "edge joins two non-HOP vertices");
                 if (uh && g->cost[e] == 0) zero_cost_hop_tail = true;
                 cost_sum += g->cost[e];
-                indeg[v + 1]++;
             }
         }
         if (g->flags & HSPF_GF_HOPCOUNT) {
@@ -637,23 +551,15 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         } else if (zero_cost_hop_tail)
             return fail(ctx, HSPF_E_NEEDS_ORACLE,
                         "zero-cost link out of a hop-counting vertex: ECMP DAG depends on pop order");
+        const Transposed t = transpose(g);
         uint32_t max_indeg = 0;
-        for (uint32_t v = 0; v < V; ++v) max_indeg = std::max(max_indeg, indeg[v + 1]);
+        for (uint32_t v = 0; v < V; ++v) max_indeg = std::max(max_indeg, t.irow[v + 1] - t.irow[v]);
         if (max_indeg >= 0xFFFFu) return fail(ctx, HSPF_E_UNSUPPORTED, "in-degree >= 65535");
 
-        // transposed CSR: in-edges of v ordered by (source, forward edge index)
-        std::vector<uint32_t> irow(V + 1, 0);
-        for (uint32_t v = 0; v < V; ++v) irow[v + 1] = irow[v] + indeg[v + 1];
-        std::vector<uint32_t> fill(irow.begin(), irow.end() - 1);
         std::vector<uint4> iedge(E);
         std::vector<uint2> fedge(E);
-        for (uint32_t u = 0; u < V; ++u)
-            for (uint32_t e = g->row_ptr[u]; e < g->row_ptr[u + 1]; ++e) {
-                const uint32_t v = g->col[e];
-                const uint32_t k = fill[v]++;
-                iedge[k] = make_uint4(u, g->cost[e], e, 0u);
-                fedge[e] = make_uint2(v, g->cost[e]);
-            }
+        for (uint32_t k = 0; k < E; ++k) iedge[k] = make_uint4(t.src[k], t.cost[k], t.fwd[k], 0u);
+        for (uint32_t e = 0; e < E; ++e) fedge[e] = make_uint2(g->col[e], g->cost[e]);
 
         // compact twins used by the jump phase when ids and costs fit 16 bits: row offsets
         // (kept in shared memory during the SSSP) and in-edges as (source | cost << 16)
@@ -664,7 +570,7 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         std::vector<uint16_t> row16(pack_rows ? V : 0);
         for (uint32_t v = 0; v < (uint32_t)row16.size(); ++v) row16[v] = (uint16_t)g->row_ptr[v];
         std::vector<uint32_t> iedge16(pack_in ? E : 0);
-        for (uint32_t k = 0; k < (uint32_t)iedge16.size(); ++k) iedge16[k] = iedge[k].x | (iedge[k].y << 16);
+        for (uint32_t k = 0; k < (uint32_t)iedge16.size(); ++k) iedge16[k] = t.src[k] | (t.cost[k] << 16);
         // ... and the same in-edge records padded per vertex to whole 16-byte quads (pad record:
         // the vertex itself with cost 0xFFFF, which can never be a parent), so the parents pass reads the usual
         // four in-edges of a vertex with one 128-bit load
@@ -673,7 +579,7 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         if (pack_in) {
             for (uint32_t v = 0; v < V; ++v) {
                 iquad_row[v] = (uint32_t)(iquad.size() / 4);
-                for (uint32_t k = irow[v]; k < irow[v + 1]; ++k) iquad.push_back(iedge16[k]);
+                for (uint32_t k = t.irow[v]; k < t.irow[v + 1]; ++k) iquad.push_back(iedge16[k]);
                 while (iquad.size() % 4) iquad.push_back(v | 0xFFFF0000u);   // pad: self-loop, never a parent
             }
             iquad_row[V] = (uint32_t)(iquad.size() / 4);
@@ -682,96 +588,45 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         for (uint32_t e = 0; e < (uint32_t)edge16.size(); ++e) edge16[e] = fedge[e].x | (fedge[e].y << 16);
 
         // quad-space image for spf_quad_kernel (quad_layout.h), when ids and costs pack
-        QuadHost QH;
-        {
-            std::vector<uint32_t> isrc(E), icost(E), ifwd(E);
-            for (uint32_t k = 0; k < E; ++k) { isrc[k] = iedge[k].x; icost[k] = iedge[k].y; ifwd[k] = iedge[k].z; }
-            QH = build_quads(V, E, g->row_ptr, g->col, g->cost, g->vflags, irow.data(), isrc.data(), icost.data(),
-                             ifwd.data(), g->delta);
-        }
-
-        auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-        const size_t o_row = 0;
-        const size_t o_edge = o_row + al((size_t)(V + 1) * 4);
-        const size_t o_irow = o_edge + al((size_t)E * 8);
-        const size_t o_iedge = o_irow + al((size_t)(V + 1) * 4);
-        const size_t o_vf = o_iedge + al((size_t)E * 16);
-        const size_t o_row16 = o_vf + al(V);
-        const size_t o_iedge16 = o_row16 + al(row16.size() * 2);
-        const size_t o_edge16 = o_iedge16 + al(iedge16.size() * 4);
-        const size_t o_iqrow = o_edge16 + al(edge16.size() * 4);
-        const size_t o_iquad = o_iqrow + al(iquad_row.size() * 4);
-        const size_t o_fq = o_iquad + al(iquad.size() * 4);
-        const size_t o_fcont = o_fq + al(QH.fq.size() * 4);
-        const size_t o_slot = o_fcont + al(QH.fcont.size() * 4);
-        const size_t o_vert = o_slot + al(QH.slot_of.size() * 2);
-        const size_t o_iq = o_vert + al(QH.vert_of.size() * 2);
-        const size_t o_imeta = o_iq + al(QH.iq.size() * 4);
-        const size_t o_fpos = o_imeta + al(QH.imeta.size() * 4);
-        const size_t o_ipos = o_fpos + al(QH.fpos.size() * 4);
-        const size_t total = o_ipos + al(QH.ipos.size() * 4);
+        const QuadHost QH = quads_of(g, t);
 
         hspf_graph *G = new hspf_graph();
+        G->has_quads = QH.eligible && !iedge16.empty();
+        BlobImage img;
+        img.add(G->d.row, g->row_ptr, V + 1);
+        img.add(G->d.edge, fedge);
+        img.add(G->d.irow, t.irow);
+        img.add(G->d.iedge, iedge);
+        img.add(G->d.vflags, g->vflags, V);
+        img.add(G->d.row16, row16, !row16.empty());
+        img.add(G->d.iedge16, iedge16, !iedge16.empty());
+        img.add(G->d.edge16, edge16, !edge16.empty());
+        img.add(G->d.iquad_row, iquad_row, !iquad_row.empty());
+        img.add(G->d.iquad, iquad, !iquad.empty());
+        // (a graph that fails late in build_quads keeps the room of the arrays built so far, zeroed)
+        auto add_quads = [&](auto &field, const auto &v) { img.add(field, QH.eligible ? v.data() : nullptr, v.size(), G->has_quads); };
+        add_quads(G->q.fq, QH.fq);
+        add_quads(G->q.fcont, QH.fcont);
+        add_quads(G->q.slot_of, QH.slot_of);
+        add_quads(G->q.vert_of, QH.vert_of);
+        add_quads(G->q.iq, QH.iq);
+        add_quads(G->q.imeta, QH.imeta);
+        add_quads(G->q.fpos, QH.fpos);
+        add_quads(G->q.ipos, QH.ipos);
         cudaError_t e = cudaSetDevice(ctx->device);
-        if (e == cudaSuccess) e = cudaMalloc(&G->blob, total);
+        if (e == cudaSuccess) e = cudaMalloc(&G->blob, img.bytes.size());
         if (e != cudaSuccess) { delete G; return cuda_fail(ctx, e, "cudaMalloc(graph)"); }
-        G->blob_bytes = total;
-        uint8_t *b = static_cast<uint8_t *>(G->blob);
-        std::vector<uint8_t> host(total, 0);
-        std::memcpy(host.data() + o_row, g->row_ptr, (size_t)(V + 1) * 4);
-        if (E) {
-            std::memcpy(host.data() + o_edge, fedge.data(), (size_t)E * 8);
-            std::memcpy(host.data() + o_iedge, iedge.data(), (size_t)E * 16);
-        }
-        std::memcpy(host.data() + o_irow, irow.data(), (size_t)(V + 1) * 4);
-        std::memcpy(host.data() + o_vf, g->vflags, V);
-        if (!row16.empty()) std::memcpy(host.data() + o_row16, row16.data(), row16.size() * 2);
-        if (!iedge16.empty()) std::memcpy(host.data() + o_iedge16, iedge16.data(), iedge16.size() * 4);
-        if (!edge16.empty()) std::memcpy(host.data() + o_edge16, edge16.data(), edge16.size() * 4);
-        if (!iquad_row.empty()) std::memcpy(host.data() + o_iqrow, iquad_row.data(), iquad_row.size() * 4);
-        if (!iquad.empty()) std::memcpy(host.data() + o_iquad, iquad.data(), iquad.size() * 4);
-        if (QH.eligible) {
-            std::memcpy(host.data() + o_fq, QH.fq.data(), QH.fq.size() * 4);
-            std::memcpy(host.data() + o_fcont, QH.fcont.data(), QH.fcont.size() * 4);
-            std::memcpy(host.data() + o_slot, QH.slot_of.data(), QH.slot_of.size() * 2);
-            std::memcpy(host.data() + o_vert, QH.vert_of.data(), QH.vert_of.size() * 2);
-            std::memcpy(host.data() + o_iq, QH.iq.data(), QH.iq.size() * 4);
-            std::memcpy(host.data() + o_imeta, QH.imeta.data(), QH.imeta.size() * 4);
-            if (E) {
-                std::memcpy(host.data() + o_fpos, QH.fpos.data(), QH.fpos.size() * 4);
-                std::memcpy(host.data() + o_ipos, QH.ipos.data(), QH.ipos.size() * 4);
-            }
-        }
-        e = cudaMemcpyAsync(b, host.data(), total, cudaMemcpyHostToDevice, ctx->stream);
+        e = cudaMemcpyAsync(G->blob, img.bytes.data(), img.bytes.size(), cudaMemcpyHostToDevice, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
         if (e != cudaSuccess) { cudaFree(G->blob); delete G; return cuda_fail(ctx, e, "graph H2D"); }
+        for (auto &b : img.bind) b(static_cast<const uint8_t *>(G->blob));
 
         G->d.V = V; G->d.E = E;
-        G->d.row = reinterpret_cast<const uint32_t *>(b + o_row);
-        G->d.edge = reinterpret_cast<const uint2 *>(b + o_edge);
-        G->d.irow = reinterpret_cast<const uint32_t *>(b + o_irow);
-        G->d.iedge = reinterpret_cast<const uint4 *>(b + o_iedge);
-        G->d.vflags = b + o_vf;
-        G->d.row16 = row16.empty() ? nullptr : reinterpret_cast<const uint16_t *>(b + o_row16);
-        G->d.iedge16 = iedge16.empty() ? nullptr : reinterpret_cast<const uint32_t *>(b + o_iedge16);
-        G->d.edge16 = edge16.empty() ? nullptr : reinterpret_cast<const uint32_t *>(b + o_edge16);
-        G->d.iquad_row = iquad_row.empty() ? nullptr : reinterpret_cast<const uint32_t *>(b + o_iqrow);
-        G->d.iquad = iquad.empty() ? nullptr : reinterpret_cast<const uint4 *>(b + o_iquad);
-        G->has_quads = QH.eligible && G->d.iedge16 != nullptr;
-        G->quad_why = QH.why;
         if (G->has_quads) {
             G->q.NQ = QH.NQ; G->q.NIQ = QH.NIQ; G->q.shift = QH.shift;
             uint32_t st = 0;
             while ((1u << st) < QH.max_ichain) ++st;
             G->q.isteps = st;
-            G->q.fq = reinterpret_cast<const uint4 *>(b + o_fq);
-            G->q.fcont = reinterpret_cast<const uint32_t *>(b + o_fcont);
-            G->q.slot_of = reinterpret_cast<const uint16_t *>(b + o_slot);
-            G->q.vert_of = reinterpret_cast<const uint16_t *>(b + o_vert);
-            G->q.iq = reinterpret_cast<const uint4 *>(b + o_iq);
-            G->q.imeta = reinterpret_cast<const uint2 *>(b + o_imeta);
-            G->q.fpos = reinterpret_cast<const uint32_t *>(b + o_fpos);
-            G->q.ipos = reinterpret_cast<const uint32_t *>(b + o_ipos);
         }
         G->d.reject_above = g->reject_above;
         G->d.saturate_at = g->saturate_at;
@@ -789,6 +644,17 @@ int hspf_graph_upload(hspf_ctx *ctx, const hspf_csr *g, hspf_graph **out) {
         G->h_vflags.assign(g->vflags, g->vflags + V);
         for (uint32_t v = 0; v < V; ++v)
             if (g->vflags[v] & (HSPF_VF_LEAF | HSPF_VF_LEAF_UNLESS_ROOT)) G->has_leaf = true;
+        // the fast path, decided once: its per-job state must fit this device's shared memory (2 KB
+        // headroom for the kernel's static shared memory)
+        if (!G->has_quads) {
+            G->why_not_fast = QH.why;
+        } else if (G->has_leaf || (g->flags & HSPF_GF_HOPCOUNT)) {
+            G->why_not_fast = "LEAF flags / hop-count mode";
+        } else {
+            G->qlay = make_quad_layout(V, QH.NQ);
+            G->fast = (size_t)G->qlay.total + 2048 <= ctx->smem_optin;
+            if (!G->fast) G->why_not_fast = "per-job state exceeds shared memory";
+        }
         *out = G;
         return HSPF_OK;
     } catch (const std::bad_alloc &) {
@@ -848,35 +714,25 @@ int hspf_sync(hspf_ctx *ctx) {
 }
 
 int hspf_run_batch_async(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const hspf_result *out) {
-    if (!ctx || !g || !jobs) return HSPF_E_INVAL;
-    if (!out) return fail(ctx, HSPF_E_INVAL, "null result");
-    return run_async_any(ctx, g, jobs, any_of(out));
+    return run_checked(ctx, g, jobs, out, true, 0);
 }
 
 int hspf_run_batch(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const hspf_result *out, uint32_t flags) {
-    if (!ctx || !g || !jobs) return HSPF_E_INVAL;
-    if (!out) return fail(ctx, HSPF_E_INVAL, "null result");
-    return run_any(ctx, g, jobs, any_of(out), flags);
+    return run_checked(ctx, g, jobs, out, false, flags);
 }
 
 int hspf_run_batch16_async(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const hspf_result16 *out) {
-    if (!ctx || !g || !jobs) return HSPF_E_INVAL;
-    if (!out) return fail(ctx, HSPF_E_INVAL, "null result");
-    return run_async_any(ctx, g, jobs, any_of(out));
+    return run_checked(ctx, g, jobs, out, true, 0);
 }
 
 int hspf_run_batch16(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs, const hspf_result16 *out, uint32_t flags) {
-    if (!ctx || !g || !jobs) return HSPF_E_INVAL;
-    if (!out) return fail(ctx, HSPF_E_INVAL, "null result");
-    return run_any(ctx, g, jobs, any_of(out), flags);
+    return run_checked(ctx, g, jobs, out, false, flags);
 }
 
 int hspf_graph_info(const hspf_graph *g, uint32_t info[8]) {
     if (!g || !info) return HSPF_E_INVAL;
-    info[0] = g->has_quads && !g->has_leaf && !(g->d.flags & HSPF_GF_HOPCOUNT) ? 1u : 0u;   // fast path / 16-bit planes available
-    info[1] = g->has_quads ? g->q.NQ : 0u;
-    info[2] = g->has_quads ? g->q.NIQ : 0u;
-    info[3] = g->has_quads ? g->q.shift : 0u;
+    info[0] = g->fast ? 1u : 0u;   // fast path / 16-bit planes available
+    info[1] = g->q.NQ; info[2] = g->q.NIQ; info[3] = g->q.shift;   // zero without a quad image
     info[4] = g->d.V; info[5] = g->d.E; info[6] = g->max_indeg; info[7] = 0;
     return HSPF_OK;
 }
@@ -885,21 +741,9 @@ int hspf_debug_quad_image(const hspf_csr *g, uint32_t hdr[8], uint32_t *fq, uint
                           uint16_t *vert_of, uint32_t *iq, uint32_t *imeta, uint32_t *fpos, uint32_t *ipos) {
     if (!g || !hdr) return HSPF_E_INVAL;
     try {
-        const uint32_t V = g->n_vertices, E = g->n_edges;
-        std::vector<uint32_t> irow(V + 1, 0), isrc(E), icost(E), ifwd(E);
-        for (uint32_t e = 0; e < E; ++e) {
-            if (g->col[e] >= V) return HSPF_E_INVAL;
-            irow[g->col[e] + 1]++;
-        }
-        for (uint32_t v = 0; v < V; ++v) irow[v + 1] += irow[v];
-        std::vector<uint32_t> fill(irow.begin(), irow.end() - 1);
-        for (uint32_t u = 0; u < V; ++u)
-            for (uint32_t e = g->row_ptr[u]; e < g->row_ptr[u + 1]; ++e) {
-                const uint32_t k = fill[g->col[e]]++;
-                isrc[k] = u; icost[k] = g->cost[e]; ifwd[k] = e;
-            }
-        QuadHost Q = build_quads(V, E, g->row_ptr, g->col, g->cost, g->vflags, irow.data(), isrc.data(), icost.data(),
-                                 ifwd.data(), g->delta);
+        for (uint32_t e = 0; e < g->n_edges; ++e)
+            if (g->col[e] >= g->n_vertices) return HSPF_E_INVAL;
+        const QuadHost Q = quads_of(g, transpose(g));
         hdr[0] = Q.eligible ? 1u : 0u; hdr[1] = Q.NQ; hdr[2] = Q.NIQ; hdr[3] = Q.shift;
         hdr[4] = Q.max_ichain; hdr[5] = Q.max_atoms; hdr[6] = 0; hdr[7] = 0;
         if (!Q.eligible) return HSPF_OK;

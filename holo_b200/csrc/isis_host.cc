@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "holo_spf_lsdb.h"
+#include "spf_one_root.h"
 
 namespace {
 constexpr uint32_t kNone = 0xFFFFFFFFu;
@@ -393,25 +394,14 @@ int hspf_isis_compute_spt(hspf_ctx *ctx, const hl_isis_level *lvl, uint64_t root
             return HSPF_OK;
         }
         const uint32_t root = it->second;
-        const uint32_t V = (uint32_t)f.ids.size();
         hspf_csr csr;
         fill_csr(f, &csr);
-        hspf_graph *g = nullptr;
-        rc = hspf_graph_upload(ctx, &csr, &g);
-        if (rc) return rc;
-        std::vector<uint32_t> dist(V);
-        std::vector<uint16_t> hops(V);
-        uint32_t status = 0;
-        hspf_jobs jobs{};
-        jobs.n_jobs = 1; jobs.roots = &root;
-        hspf_result res{};
-        res.dist = dist.data(); res.hops = hops.data(); res.nh_words = 4; res.job_status = &status;
-        rc = hspf_run_batch(ctx, g, &jobs, &res, 0);
-        hspf_graph_free(ctx, g);
+        hspf::OneRootPlanes p;
+        rc = hspf::run_one_root(ctx, csr, root, 4, false, p);
         // first-hop atom overflow is irrelevant here: the Vec is rebuilt from parents
-        if (rc == HSPF_E_JOB_STATUS && !(status & ~HSPF_JS_TOO_MANY_ATOMS)) rc = HSPF_OK;
+        if (rc == HSPF_E_JOB_STATUS && !(p.status & ~HSPF_JS_TOO_MANY_ATOMS)) rc = HSPF_OK;
         if (rc) return rc;
-        return spt_from_planes(f, root, dist.data(), hops.data(), 0, nullptr, nullptr, out);
+        return spt_from_planes(f, root, p.dist.data(), p.hops.data(), 0, nullptr, nullptr, out);
     } catch (const std::bad_alloc &) { return HSPF_E_NOMEM; } catch (...) { return HSPF_E_INVAL; }
 }
 
@@ -781,24 +771,13 @@ extern "C" int hspf_isis_compute_routes(hspf_ctx *ctx, const hl_isis_instance *i
             int rc = topology_flat(in, mt_id, f, root, have_root);
             if (rc) return rc;
             if (!have_root) continue;
-            const uint32_t V = (uint32_t)f.ids.size();
             hspf_csr csr;
             fill_csr(f, &csr);
-            hspf_graph *g = nullptr;
-            rc = hspf_graph_upload(ctx, &csr, &g);
+            hspf::OneRootPlanes p;
+            rc = hspf::run_one_root(ctx, csr, root, 4, false, p);
+            if (rc == HSPF_E_JOB_STATUS && !(p.status & ~HSPF_JS_TOO_MANY_ATOMS)) rc = HSPF_OK;
             if (rc) return rc;
-            std::vector<uint32_t> dist(V);
-            std::vector<uint16_t> hops(V);
-            uint32_t status = 0;
-            hspf_jobs jobs{};
-            jobs.n_jobs = 1; jobs.roots = &root;
-            hspf_result res{};
-            res.dist = dist.data(); res.hops = hops.data(); res.nh_words = 4; res.job_status = &status;
-            rc = hspf_run_batch(ctx, g, &jobs, &res, 0);
-            hspf_graph_free(ctx, g);
-            if (rc == HSPF_E_JOB_STATUS && !(status & ~HSPF_JS_TOO_MANY_ATOMS)) rc = HSPF_OK;
-            if (rc) return rc;
-            rc = topology_routes(in, f, mt_id, root, dist.data(), hops.data(), rib);
+            rc = topology_routes(in, f, mt_id, root, p.dist.data(), p.hops.data(), rib);
             if (rc) return rc;
         }
         return emit_rib(rib, out);

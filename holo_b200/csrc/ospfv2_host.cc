@@ -21,6 +21,7 @@
 
 #include "holo_spf_lsdb.h"
 #include "route_cells.h"
+#include "spf_one_root.h"
 
 namespace {
 
@@ -674,7 +675,6 @@ int hspf_ospfv2_run_area(hspf_ctx *ctx, const hl_ospfv2_area *a, hl_ospfv2_resul
         if (rit == f.rtr_vertex.end()) return HSPF_OK;   // SpfRootNotFound: logged, nothing computed
         out->root_found = 1;
         const uint32_t root = rit->second;
-        const uint32_t V = (uint32_t)f.ids.size();
 
         // ---- SPT on the device ---------------------------------------------------------
         hspf_csr csr;
@@ -683,23 +683,10 @@ int hspf_ospfv2_run_area(hspf_ctx *ctx, const hl_ospfv2_area *a, hl_ospfv2_resul
         hspf_atom_count(&csr, root, &n_atoms);
         const uint32_t nhw = std::max(1u, (n_atoms + 63) / 64);
         if (nhw > 4) return HSPF_E_UNSUPPORTED;   // > 256 first-hop atoms: caller's CPU path
-        hspf_graph *g = nullptr;
-        rc = hspf_graph_upload(ctx, &csr, &g);
-        if (rc) return rc;
-        std::vector<uint32_t> dist(V);
-        std::vector<uint16_t> hops(V);
-        std::vector<uint64_t> nh((size_t)V * nhw);
-        uint32_t status = 0;
-        hspf_jobs jobs{};
-        jobs.n_jobs = 1;
-        jobs.roots = &root;
-        hspf_result res{};
-        res.dist = dist.data(); res.hops = hops.data(); res.nh_mask = nh.data(); res.nh_words = nhw;
-        res.job_status = &status;
-        rc = hspf_run_batch(ctx, g, &jobs, &res, 0);
-        hspf_graph_free(ctx, g);
+        hspf::OneRootPlanes p;
+        rc = hspf::run_one_root(ctx, csr, root, nhw, true, p);
         if (rc) return rc;   // includes HSPF_E_JOB_STATUS (saturation): caller's CPU path
-        return area_from_planes(f, a, root, dist.data(), hops.data(), nh.data(), nhw, out);
+        return area_from_planes(f, a, root, p.dist.data(), p.hops.data(), p.nh.data(), nhw, out);
     } catch (const std::bad_alloc &) {
         return HSPF_E_NOMEM;
     } catch (...) {

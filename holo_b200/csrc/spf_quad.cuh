@@ -22,9 +22,10 @@
 //              jump terminals (the scheme of spf_kernel.cuh phase 3J), 16 first-hop atoms
 //              per pass, up to four passes (64 atoms).
 //
-// Eligibility (checked by the host, hspf_capi.cu): packed ids and costs (V, quads < 65535,
-// costs <= 65534, degrees <= 128), no LEAF vertex flags, no hop-count mode, one next-hop
-// word.  Everything else runs spf_batch_kernel.
+// Eligibility (decided by the host at graph upload, hspf_capi.cu): packed ids and costs (V,
+// quads < 65535, costs <= 65534, degrees <= 128), no LEAF vertex flags, no hop-count mode,
+// per-job state within shared memory; and one next-hop word.  Everything else runs
+// spf_batch_kernel.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -37,6 +38,7 @@ constexpr uint32_t kJsInvalid = 8u;   // HSPF_JS_INVALID
 constexpr uint32_t kJsInternal = 16u; // HSPF_JS_INTERNAL: a loop bound that cannot be reached was reached
 constexpr uint32_t kJsNarrow = 32u;   // HSPF_JS_NARROW: the job's result does not fit 16-bit planes
 constexpr int kQMaxRoot = 64;         // non-HOP root neighbours tracked (>= 64 atoms is refused anyway)
+constexpr int kQuadThreads = 512;     // CTA size, the fastest of the sweep in profiles/r2_kernel_history.md
 
 struct QuadDev {
     uint32_t NQ, NIQ, shift, isteps;
@@ -51,8 +53,7 @@ struct QuadDev {
 };
 
 struct QuadLayout {   // byte offsets into dynamic shared memory
-    uint32_t dist, queue, ring, cont, h0, ecmp, elist, total;
-    uint32_t qcap;    // queue capacity (entries)
+    uint32_t dist, ring, cont, h0, ecmp, elist, total;
 };
 
 struct QuadArgs {
@@ -71,7 +72,6 @@ struct QuadArgs {
     uint64_t *out_nh;
     uint32_t *out_status;
     uint32_t *job_counter;
-    uint32_t sub_rounds;        // visits of a warp to its bitmap chunk per barrier-separated round (>= 1)
     uint32_t narrow;            // 1: 16-bit result planes (hspf_result16): out_dist / out_fp / out_nh point at u16 arrays
     // Fused exchange (multi-GPU, 16-bit planes): the result writer also stores the planes the
     // consumers need (dist, hops, nh_mask, job status) into this rank's slot on every peer GPU,
@@ -83,16 +83,14 @@ struct QuadArgs {
     unsigned long long *prof;   // optional [gridDim][16] cycle counters
 };
 
-// `threads` = CTA size: the jump words are padded to a multiple of 4 * threads (unrolled rounds
-// without bounds checks).
-inline QuadLayout make_quad_layout(uint32_t V, uint32_t NQ, uint32_t qcap, uint32_t threads) {
+// The jump words are padded to a multiple of 4 * kQuadThreads (unrolled rounds without bounds checks).
+inline QuadLayout make_quad_layout(uint32_t V, uint32_t NQ) {
     QuadLayout L{};
     auto al = [](size_t x) { return (uint32_t)((x + 15) / 16 * 16); };
     const uint32_t nbv = (V + 31) / 32, nbw = (NQ / 32 + 1u) & ~1u;   // bitmap rows: an even number of words
-    const uint32_t Vp = (V + 4 * threads - 1) / (4 * threads) * (4 * threads);
+    const uint32_t Vp = (V + 4 * kQuadThreads - 1) / (4 * kQuadThreads) * (4 * kQuadThreads);
     uint32_t o = 0;
     L.dist = o; o += al((size_t)NQ * 4);
-    L.queue = o; o += al((size_t)qcap * 4);
     // phase 3: jump words u32[Vp] over dist, ECMP vertex list u16[V] behind them
     L.elist = al((size_t)Vp * 4);
     if (L.elist + al((size_t)V * 2) > o) o = L.elist + al((size_t)V * 2);
@@ -101,11 +99,11 @@ inline QuadLayout make_quad_layout(uint32_t V, uint32_t NQ, uint32_t qcap, uint3
     L.h0 = o; o += al((size_t)nbv * 4);
     L.ecmp = o; o += al((size_t)nbv * 4);
     L.total = o;
-    L.qcap = qcap;
     return L;
 }
 
 struct QSmall {
+    long long t_mark;     // phase profile clock of thread 0 (here, not in a register held through the kernel)
     uint32_t cnt[2];
     uint32_t wake;        // epoch: bumped by a working warp that sees plenty of work while others sleep
     uint32_t status;
@@ -121,13 +119,14 @@ struct QSmall {
     do {                                                                         \
         if (a.prof && tid == 0) {                                                \
             const long long now_ = clock64();                                    \
-            a.prof[(size_t)blockIdx.x * 16 + (k)] += (unsigned long long)(now_ - t_mark); \
-            t_mark = now_;                                                       \
+            a.prof[(size_t)blockIdx.x * 16 + (k)] += (unsigned long long)(now_ - S.t_mark); \
+            S.t_mark = now_;                                                     \
         }                                                                        \
     } while (0)
 
-template <int T, bool kOv>
-__global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
+template <bool kOv>
+__global__ void __launch_bounds__(kQuadThreads, 3) spf_quad_kernel(const QuadArgs a) {
+    constexpr int T = kQuadThreads;
     extern __shared__ __align__(16) uint8_t qsm[];
     __shared__ QSmall S;
 
@@ -137,10 +136,8 @@ __global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
     const uint32_t V = g.V, NQ = Q.NQ, NBW = NQ >> 5, nbv = (V + 31) >> 5;
     const uint32_t NBWp = (NBW + 1u) & ~1u;     // bitmap row stride: an even number of words
     const uint32_t tid = threadIdx.x, lane = tid & 31;
-    const uint32_t qcap = L.qcap;
 
     uint32_t *dist = reinterpret_cast<uint32_t *>(qsm + L.dist);
-    uint32_t *queue = reinterpret_cast<uint32_t *>(qsm + L.queue);   // entries: quad | first quad of its chain << 16
     uint32_t *ring = reinterpret_cast<uint32_t *>(qsm + L.ring);     // frontier bitmaps, word w of bucket b at [w * 4 + (b & 3)]
     uint32_t *cont_s = reinterpret_cast<uint32_t *>(qsm + L.cont);
     uint32_t *h0bm = reinterpret_cast<uint32_t *>(qsm + L.h0);
@@ -148,7 +145,7 @@ __global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
     uint32_t *word = dist;                                   // phase 3
     uint16_t *elist = reinterpret_cast<uint16_t *>(qsm + L.elist);
 
-    long long t_mark = clock64();
+    if (tid == 0) S.t_mark = clock64();
 
     // once per CTA: chain-continuation bits
     for (uint32_t w = tid; w < NBWp; w += T) cont_s[w] = (w < NBW) ? Q.fcont[w] : 0u;
@@ -338,15 +335,13 @@ __global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
             // finds its quad by itself — owner word by binary search over the scanned counts
             // (shuffles), then the k-th set bit of that word — so all lanes work in every pass,
             // whatever the distribution of bits over the words, and the quad goes straight from the
-            // lane's registers into the relaxation: no queue, no CTA-wide scan.  A warp visits its
-            // chunk `a.sub_rounds` times per round; one CTA barrier per round; the bucket is
-            // finished by a round that claimed nothing.
+            // lane's registers into the relaxation: no queue, no CTA-wide scan.  One CTA barrier per
+            // round; the bucket is finished by a round that claimed nothing.
             constexpr uint32_t kWarps_ = T / 32;
             const uint32_t warp = tid >> 5;
             // chunk = the bitmap words of one claim (one per lane): sized so that every warp owns one
             const uint32_t cw = min(32u, (NBWp + kWarps_ - 1) / kWarps_);
             const uint32_t nchunks = (NBWp + cw - 1) / cw;
-            const uint32_t sub_rounds = a.sub_rounds;
             // output index t of a claimed chunk -> queue-less entry (quad | first quad of its chain << 16)
             auto pick = [&](uint32_t t, uint32_t incl, uint32_t bits, uint32_t meta, uint32_t C) -> uint32_t {
                 uint32_t lo = 0;      // owner = number of lanes whose inclusive count is <= t
@@ -378,46 +373,44 @@ __global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
                 if (guard > (1u << 24)) { if (tid == 0) atomicOr(&S.status, kJsInternal); break; }   // defensive
                 uint32_t *bm = ring + (cur & 3u);
                 int claimed = 0;
-                for (uint32_t sr = 0; sr < sub_rounds; ++sr) {
-                    for (uint32_t c = warp; c < nchunks; c += kWarps_) {
-                        const uint32_t w = c * cw + lane;
-                        const bool mine = lane < cw && w < NBWp;
-                        uint32_t bits = mine ? *reinterpret_cast<volatile uint32_t *>(&bm[w << 2]) : 0u;
-                        if (!__any_sync(0xffffffffu, bits != 0)) continue;
-                        claimed = 1;
-                        uint32_t C = 0;
-                        if (bits) {
-                            bits = atomicExch(&bm[w << 2], 0u);
-                            C = cont_s[w];
-                            uint32_t m = bits;
-                            while ((m = (m << 1) & C) != 0) bits |= m;      // the other quads of a multi-quad vertex
-                        }
-                        const uint32_t cnt = __popc(bits);
-                        uint32_t incl = cnt;
+                for (uint32_t c = warp; c < nchunks; c += kWarps_) {
+                    const uint32_t w = c * cw + lane;
+                    const bool mine = lane < cw && w < NBWp;
+                    uint32_t bits = mine ? *reinterpret_cast<volatile uint32_t *>(&bm[w << 2]) : 0u;
+                    if (!__any_sync(0xffffffffu, bits != 0)) continue;
+                    claimed = 1;
+                    uint32_t C = 0;
+                    if (bits) {
+                        bits = atomicExch(&bm[w << 2], 0u);
+                        C = cont_s[w];
+                        uint32_t m = bits;
+                        while ((m = (m << 1) & C) != 0) bits |= m;      // the other quads of a multi-quad vertex
+                    }
+                    const uint32_t cnt = __popc(bits);
+                    uint32_t incl = cnt;
 #pragma unroll
-                        for (int o = 1; o < 32; o <<= 1) {
-                            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-                            if ((int)lane >= o) incl += t;
-                        }
-                        const uint32_t n = __shfl_sync(0xffffffffu, incl, 31);
-                        const uint32_t meta = (incl - cnt) | (w << 16);
-                        if (a.prof && lane == 0) atomicAdd(&a.prof[(size_t)blockIdx.x * 16 + 12], (unsigned long long)n);
-                        // two quads of a lane in flight
-                        for (uint32_t t0 = 0; t0 < n; t0 += 64) {
-                            const uint32_t ta = t0 + lane, tb = ta + 32;
-                            const bool hb = t0 + 32 < n;                       // warp-uniform
-                            const uint32_t e0 = pick(ta, incl, bits, meta, C);
-                            const uint32_t e1 = hb ? pick(tb, incl, bits, meta, C) : 0u;
-                            const uint32_t du0 = (ta < n) ? dist[e0 >> 16] : kInf;     // the chain owner's distance
-                            const uint32_t du1 = (hb && tb < n) ? dist[e1 >> 16] : kInf;
-                            // a mark is stale when the vertex was settled in an earlier bucket
-                            const bool l0 = (du0 >> sh) == cur, l1 = (du1 >> sh) == cur;
-                            uint4 r0 = make_uint4(0u, 0u, 0u, 0u), r1 = r0;
-                            if (l0) r0 = __ldg(&Q.fq[e0 & 0xFFFFu]);
-                            if (l1) r1 = __ldg(&Q.fq[e1 & 0xFFFFu]);
-                            if (l0) relax(e0 & 0xFFFFu, e0 >> 16, du0, r0);
-                            if (l1) relax(e1 & 0xFFFFu, e1 >> 16, du1, r1);
-                        }
+                    for (int o = 1; o < 32; o <<= 1) {
+                        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+                        if ((int)lane >= o) incl += t;
+                    }
+                    const uint32_t n = __shfl_sync(0xffffffffu, incl, 31);
+                    const uint32_t meta = (incl - cnt) | (w << 16);
+                    if (a.prof && lane == 0) atomicAdd(&a.prof[(size_t)blockIdx.x * 16 + 12], (unsigned long long)n);
+                    // two quads of a lane in flight
+                    for (uint32_t t0 = 0; t0 < n; t0 += 64) {
+                        const uint32_t ta = t0 + lane, tb = ta + 32;
+                        const bool hb = t0 + 32 < n;                       // warp-uniform
+                        const uint32_t e0 = pick(ta, incl, bits, meta, C);
+                        const uint32_t e1 = hb ? pick(tb, incl, bits, meta, C) : 0u;
+                        const uint32_t du0 = (ta < n) ? dist[e0 >> 16] : kInf;     // the chain owner's distance
+                        const uint32_t du1 = (hb && tb < n) ? dist[e1 >> 16] : kInf;
+                        // a mark is stale when the vertex was settled in an earlier bucket
+                        const bool l0 = (du0 >> sh) == cur, l1 = (du1 >> sh) == cur;
+                        uint4 r0 = make_uint4(0u, 0u, 0u, 0u), r1 = r0;
+                        if (l0) r0 = __ldg(&Q.fq[e0 & 0xFFFFu]);
+                        if (l1) r1 = __ldg(&Q.fq[e1 & 0xFFFFu]);
+                        if (l0) relax(e0 & 0xFFFFu, e0 >> 16, du0, r0);
+                        if (l1) relax(e1 & 0xFFFFu, e1 >> 16, du1, r1);
                     }
                 }
                 if (a.prof && tid == 0) a.prof[(size_t)blockIdx.x * 16 + 7] += 1;
@@ -450,9 +443,9 @@ __global__ void __launch_bounds__(T, 3) spf_quad_kernel(const QuadArgs a) {
                 for (uint32_t k = 0; k < S.n_roottab; ++k) {
                     const uint32_t N = S.rt_target[k], nb = S.rt_base[k];
                     if (atom < nb || atom >= nb + (g.row[N + 1] - g.row[N])) continue;
-                    bool first = true;   // parallel root edges: only the first one's range is used
-                    for (uint32_t q = 0; q < k; ++q) first = first && S.rt_target[q] != N;
-                    if (first && hops0(N)) { u = N; e = g.row[N] + (atom - nb); }
+                    uint32_t q = 0;      // parallel root edges: only the first one's range is used
+                    while (q < k && S.rt_target[q] != N) ++q;
+                    if (q == k && hops0(N)) { u = N; e = g.row[N] + (atom - nb); }
                     break;
                 }
             }

@@ -247,7 +247,8 @@ int hspf_run_batch16(hspf_ctx *ctx, const hspf_graph *g, const hspf_jobs *jobs,
                      const hspf_result16 *out, uint32_t flags);
 int hspf_run_batch16_async(hspf_ctx *ctx, const hspf_graph *g,
                            const hspf_jobs *jobs, const hspf_result16 *out);
-/* info = {1 if the packed fast path (and so hspf_run_batch16) serves this graph, forward quads,
+/* info = {1 if the packed fast path (and so hspf_run_batch16) serves this graph: packed quad image,
+ * no LEAF flags, no hop-count mode, per-job state within the device's shared memory; forward quads,
  * in-quads, log2 of the bucket width, n_vertices, n_edges, largest in-degree, 0}. */
 int hspf_graph_info(const hspf_graph *g, uint32_t info[8]);
 /* The ctx's cudaStream_t (as void*) so callers can record CUDA events on it. */
@@ -281,6 +282,16 @@ int hspf_ctx_reserve_sms(hspf_ctx *ctx, int n_sms);
  * compaction, barrier), 12 frontier entries, 13-15 jump phase: hop rounds, next-hop rounds,
  * ECMP sweeps (Kahn path: round internals).  `out` may be NULL. */
 int hspf_debug_phase_profile(hspf_ctx *ctx, int enable, uint64_t out[16]);
+
+/* Test aid: which kernel the batches of this ctx run.  HSPF_PATH_AUTO (the default) takes the packed
+ * fast path wherever it serves the graph (hspf_graph_info) and one next-hop word is asked for;
+ * HSPF_PATH_GENERAL always runs the general kernel, HSPF_PATH_GENERAL_KAHN the general kernel
+ * without its pointer-jumping next-hop phase.  Every path gives the same planes; 16-bit planes
+ * need HSPF_PATH_AUTO. */
+#define HSPF_PATH_AUTO 0
+#define HSPF_PATH_GENERAL 1
+#define HSPF_PATH_GENERAL_KAHN 2
+int hspf_debug_set_path(hspf_ctx *ctx, int path);
 
 /* Debug / test aid (host only, no CUDA call): build the quad-space image the fast-path kernel
  * reads (holo_b200/csrc/quad_layout.h) and copy it out.  hdr = {eligible, n_fwd_quads, n_in_quads,

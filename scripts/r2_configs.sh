@@ -11,10 +11,6 @@ if [ -z "$SKIP_DEFAULT" ]; then
 echo "== bench default (C2)" >> $log
 timeout 400 python bench.py > gpurun_out/${tag}_C2.json 2> gpurun_out/${tag}_C2.err || { echo FAILED >> $log; tail -5 gpurun_out/${tag}_C2.err >> $log; }
 fi
-for ch in ${CHUNKS:-}; do
-  echo "== e2e chunk $ch" >> $log
-  HSPF_E2E_CHUNK=$ch timeout 200 python scripts/bench_brief.py --steps 10 --warmup 3 --no-cpu-baseline --no-e2e-variants >> $log 2>&1
-done
 for c in ${CFGS:-C1 C3 C4 C5}; do
   echo "== bench $c" >> $log
   timeout 500 python bench.py --config $c --steps 5 --warmup 3 ${CFG_ARGS:---cpu-seconds 4} > gpurun_out/${tag}_$c.json 2> gpurun_out/${tag}_$c.err || { echo FAILED >> $log; tail -5 gpurun_out/${tag}_$c.err >> $log; }

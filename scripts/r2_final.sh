@@ -1,5 +1,5 @@
 #!/bin/bash
-# Round-2 acceptance on one B200 (under gpurun): whole -m gpu suite, smoke(), e2e piece sweep, the
+# Round-2 acceptance on one B200: whole -m gpu suite, smoke(), the
 # default bench line, the ncu launch list of the same command and one `ncu --set full` capture.
 mkdir -p gpurun_out
 tag=${1:-r2final}
@@ -8,9 +8,6 @@ log=gpurun_out/${tag}.log
 step() { echo "== $1" >> $log; shift; timeout "$@" >> $log 2>&1; rc=$?; if [ $rc -ne 0 ]; then echo "STEP FAILED rc=$rc" >> $log; fi; }
 step "pytest -m gpu" 600 python -m pytest tests -q -m gpu
 step "smoke" 120 python __graft_entry__.py smoke
-for pc in ${PIECES:-2 3 6}; do
-  HSPF_E2E_PIECES=$pc step "e2e pieces=$pc" 100 python scripts/bench_brief.py --steps 10 --warmup 3 --no-cpu-baseline --no-e2e-variants
-done
 echo "== default bench" >> $log
 timeout 400 python bench.py > gpurun_out/${tag}_bench.json 2> gpurun_out/${tag}_bench.err; tail -c 400 gpurun_out/${tag}_bench.json >> $log
 echo "== reference arm" >> $log

@@ -187,6 +187,24 @@ def test_large_vertex_count_uses_global_state(ctx):
     g.free()
 
 
+def test_quad_image_beyond_shared_memory_runs_the_general_kernel(ctx):
+    """40 000 routers have a quad image, but its per-job state (~280 KB) exceeds shared memory: the
+    graph is not on the fast path, and a host-pointer batch big enough for the pipelined copy-back
+    (>= 256 jobs) runs the general kernel and returns."""
+    from holo_b200.capi import quad_image
+    t = synth.random_topology(40000, 80000, synth.SEED_BASE + 41)
+    csr = synth.topology_csr(t)
+    assert quad_image(csr).eligible
+    g = ctx.upload(csr)
+    assert not ctx.graph_info(g)["fast_path"]
+    roots = np.arange(0, 40000, 156, dtype=np.uint32)[:256]
+    assert len(roots) == 256
+    res = ctx.run(g, roots)
+    for j in (0, 128, 255):
+        check(res, j, pyoracle.csr_spf(csr, int(roots[j])))
+    g.free()
+
+
 def test_edge_cases_through_the_abi(ctx):
     # single isolated vertex
     csr = Csr(np.asarray([0, 0], np.uint32), np.zeros(0, np.uint32), np.zeros(0, np.uint32),
@@ -247,10 +265,10 @@ def test_many_first_hop_atoms_need_more_words(ctx):
     (400, 1200, 8, dict(cost_choices=[5]), False),              # all-equal costs: ECMP under ECMP
     (3000, 12000, 9, dict(cost_choices=[10, 20, 30], lan_fraction=0.05), False),
 ])
-def test_jump_and_kahn_next_hop_phases_agree_with_oracle(ctx, monkeypatch, V, E, seed, kw, isis):
+def test_jump_and_kahn_next_hop_phases_agree_with_oracle(ctx, V, E, seed, kw, isis):
     """One next-hop word, no overrides: the engine propagates next hops by pointer jumping
-    when the root has at most 32 first-hop atoms and by the Kahn push otherwise (or when
-    HSPF_NO_JUMP is set).  Both must give the oracle's planes."""
+    when the root has at most 32 first-hop atoms and by the Kahn push otherwise (or on the
+    "general_kahn" path).  Both must give the oracle's planes."""
     t = synth.random_topology(V, E, synth.SEED_BASE + seed, **kw)
     csr = synth.topology_csr(t, isis=isis)
     g = ctx.upload(csr)
@@ -261,13 +279,9 @@ def test_jump_and_kahn_next_hop_phases_agree_with_oracle(ctx, monkeypatch, V, E,
     assert len(ok) > len(roots) // 2
     # three device paths: the quad-space kernel (default), and spf_batch_kernel with the
     # pointer-jumping and the Kahn next-hop phase
-    for no_quad, no_jump in ((False, False), (True, False), (True, True)):
-        for name, on in (("HSPF_NO_QUAD", no_quad), ("HSPF_NO_JUMP", no_jump)):
-            if on:
-                monkeypatch.setenv(name, "1")
-            else:
-                monkeypatch.delenv(name, raising=False)
-        res = ctx.run(g, roots, nh_words=1)   # a root that ran out of atoms only flags its own job
+    for path in ("auto", "general", "general_kahn"):
+        with ctx.path(path):
+            res = ctx.run(g, roots, nh_words=1)   # a root that ran out of atoms only flags its own job
         for j in ok:
             check(res, j, refs[j])
         for j, ref in enumerate(refs):
@@ -353,11 +367,8 @@ def test_device_pointer_jobs_are_validated_on_the_device(ctx):
     t = synth.random_topology(200, 900, synth.SEED_BASE + 22)
     csr = synth.topology_csr(t)
     V = csr.n_vertices
-    for no_quad in (False, True):
-        import os
-        if no_quad:
-            os.environ["HSPF_NO_QUAD"] = "1"
-        try:
+    for path in ("auto", "general"):
+        with ctx.path(path):
             g = ctx.upload(csr)
             roots = torch.tensor([0, V + 7, 5, 0xFFFFFFF], dtype=torch.int32, device="cuda")
             n = 4
@@ -386,8 +397,6 @@ def test_device_pointer_jobs_are_validated_on_the_device(ctx):
             assert np.array_equal(d[2], pyoracle.csr_spf(csr, 5)["dist"])
             assert (bufs["dist"][1] == -7).all()          # skipped job: planes untouched
             g.free()
-        finally:
-            os.environ.pop("HSPF_NO_QUAD", None)
 
 
 def test_reserved_sms_shrink_the_grid_and_small_batches_still_run(ctx):
@@ -413,7 +422,6 @@ def test_update_costs_in_place_equals_a_fresh_upload(ctx, shape):
     """hspf_graph_update_costs patches every cost-bearing array of the device image (CSR, transpose, packed
     twins, quad-space records): a batch on the patched graph gives the planes of a fresh upload of the
     modified CSR, on the fast path, on the general path (u32 costs) and with transit networks."""
-    import os
     from holo_b200 import capi
     kw = dict(lans=dict(lan_fraction=0.1)).get(shape, {})
     t = synth.random_topology(400, 1800, synth.SEED_BASE + 61, **kw)
@@ -443,11 +451,8 @@ def test_update_costs_in_place_equals_a_fresh_upload(ctx, shape):
     for j in (0, 17, 39):
         ref = pyoracle.csr_spf_heap(csr2, int(roots[j]), nh_words=1)
         assert np.array_equal(got.dist[j], ref["dist"]) and np.array_equal(got.nh_mask[j].reshape(-1), ref["nh_mask"].reshape(-1))
-    os.environ["HSPF_NO_QUAD"] = "1"                            # the general kernel reads the other copies
-    try:
+    with ctx.path("general"):                                   # the general kernel reads the other copies
         alt = ctx.run(g, roots)
-    finally:
-        del os.environ["HSPF_NO_QUAD"]
     for name in ("dist", "hops", "first_parent", "n_parents", "nh_mask"):
         assert np.array_equal(getattr(alt, name), getattr(want, name)), name
     # refusals leave the graph as it is
